@@ -61,6 +61,8 @@ def parse_args():
     ap.add_argument("--no-kernels", action="store_true", help="skip the K1/K2 side measurements")
     ap.add_argument("--no-configs", action="store_true", help="skip the other BASELINE configurations")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling sub-record (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (traces, final graphs, counters) as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -373,6 +375,8 @@ def run_ours(a):
             dist.barrier()
             dist.destroy_process_group()
         return
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, step_outputs(r0, world))
 
     peaks = {}
     pk_path = os.path.join(ROOT, "MEASURED_PEAKS.json")
@@ -495,6 +499,67 @@ def run_ours(a):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+TRACE_COLS = ("iter", "ChangedNode", "movetype", "globalLL", "additions", "deletions", "FN", "FP")
+COUNTERS = ("uniforms", "valid_iters", "proposed", "reject", "n_nonpd", "total_edges")
+DUMP_LIMIT = 64 << 20   # bytes
+
+
+def step_outputs(r0, world):
+    """What one resident step hands its caller, one entry per chain: the trace columns (a list of the chains'
+    rows; chains write different numbers of rows) and, on one GPU, the final graphs and chain counters (chains
+    on axis 0).  With N > 1 the traces of all chains, which every rank holds after the all-gather."""
+    if world > 1:
+        from bayesnetworks_b200.dist import INT_COLUMNS
+        o = r0["out"]
+        n_rows = o["n_rows"].cpu().numpy()
+        ints = o["ints"].cpu().numpy()   # [chains, capacity, 7]
+        gll = o["gll"].cpu().numpy()
+        out = {"n_rows": n_rows, "trace_globalLL": [gll[c, :r] for c, r in enumerate(n_rows)]}
+        for i, k in enumerate(INT_COLUMNS):
+            out["trace_" + k] = [ints[c, :r, i] for c, r in enumerate(n_rows)]
+        return out
+    res = r0["results"]
+    out = {"n_rows": np.array([len(r.trace["iter"]) for r in res])}
+    for k in TRACE_COLS:
+        out["trace_" + k] = [r.trace[k] for r in res]
+    out["final_parents"] = np.stack([r.final_parents for r in res])
+    out["final_npar"] = np.stack([r.final_npar for r in res])
+    for k in COUNTERS:
+        out[k] = np.array([getattr(r, k) for r in res])
+    return out
+
+
+def dump_outputs(path, arrays):
+    """Write `arrays` as path/<name>.npy in float64.  Each value has one entry per chain: an array with chains on
+    axis 0, or a list of per-chain rows (trace columns), written end to end in chain order (n_rows.npy splits
+    them).  Above DUMP_LIMIT bytes in all, a fixed seeded sample of whole chains is written; chain_index.npy
+    says which.  When no single chain fits, the first chain of that sample is written with a seeded sample of
+    its trace rows; row_index.npy says which (n_rows.npy keeps the chain's full row count)."""
+    n = len(arrays["n_rows"])
+    arrays = dict(arrays, chain_index=np.arange(n))
+    size = np.zeros(n)
+    for v in arrays.values():
+        size += [8 * np.size(x) for x in v]
+    order = np.random.default_rng(0).permutation(n) if size.sum() > DUMP_LIMIT else np.arange(n)
+    idx = np.sort(order[np.cumsum(size[order]) <= DUMP_LIMIT])
+    if n and not len(idx):
+        c = int(order[0])
+        cols = [k for k, v in arrays.items() if isinstance(v, list)]
+        n_r = len(arrays[cols[0]][c])
+        fixed = size[c] - 8 * len(cols) * n_r   # bytes of the chain outside its trace rows
+        keep = min(n_r, max(0, int(DUMP_LIMIT - fixed) // (8 * (len(cols) + 1))))   # (+ row_index)
+        rows = np.sort(np.random.default_rng(0).choice(n_r, keep, replace=False))
+        arrays.update({k: {c: np.asarray(arrays[k][c])[rows]} for k in cols}, row_index={c: rows})
+        idx = np.array([c])
+    os.makedirs(path, exist_ok=True)
+    for name, v in arrays.items():
+        if isinstance(v, (list, dict)):   # per-chain rows (a dict: only the sampled chain's)
+            out = np.concatenate([np.zeros(0)] + [np.ravel(v[i]) for i in idx])
+        else:
+            out = np.asarray(v)[idx]
+        np.save(os.path.join(path, name + ".npy"), out.astype(np.float64))
 
 
 def config5(a, dev, rank, world):

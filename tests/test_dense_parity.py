@@ -82,21 +82,6 @@ def test_port_pinned_to_reference_dense(oracle, dense, name):
     assert list(o.proposed) == list(dense[f"{name}_proposed"])
 
 
-def test_compiled_reference_regenerates_fixture(dense):
-    """Where oracle/_ref exists (the build container) the fixture is reproducible from it."""
-    from oracle.oracle import RNG_WH, Ref, have_ref
-    if not have_ref():
-        pytest.skip("oracle/_ref not built here")
-    name = "p1000_sat"
-    _, P, phi, omega, seeds = CASES[name]
-    X, g, nt = inputs_for(P, dense)
-    r = Ref().main_fun(X, g.source, g.target, nt, MaxPar=MAX_PAR, phi=phi, omega=omega, N=N_ITER, output=OUTPUT,
-                       rng_kind=RNG_WH, seeds=seeds)
-    for k in COLS:
-        assert np.array_equal(getattr(r, k), dense[f"{name}_{k}"]), k
-    assert r.uniforms == int(dense[f"{name}_uniforms"])
-
-
 @pytest.mark.parametrize("name", ["p1000_mid", "p1024_sat", "p1025_sat"])
 def test_chain_core_host_build_dense(emu_lib, dense, name):
     """The chain core compiled for the host (one-lane warp) on the same cases: round logic,

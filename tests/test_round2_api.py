@@ -2,9 +2,12 @@
 graphs denser than MaxPar, a defined InitialNetwork = 1, R's stream state in and out, degenerate
 (collinear) data.  CPU tests pin the oracle and the host build of the chain core; `gpu` tests go
 through the C ABI."""
+import os
+
 import numpy as np
 import pytest
 
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 INT_COLS = ("iter", "ChangedNode", "movetype", "additions", "deletions", "FN", "FP")
 
 
@@ -54,11 +57,16 @@ def synthetic(P, N, max_par, seed):
 # ---------------------------------------------------------------------------
 def test_oracle_supplied_graph_denser_than_maxpar_matches_reference(oracle, dataset):
     """InitialNetwork = 2: the supplied graph only feeds simEdge / NsimEdges (src/network.h:138-146,
-    164-169), so a node with 8 prior parents and MaxPar = 3 is a legal reference run."""
+    164-169), so a node with 8 prior parents and MaxPar = 3 is a legal reference run.  The stored trace
+    is tests/golden/denser_maxpar3.npz (tests/golden/make_golden_denser.py; its `source` says what made
+    it); where oracle/_ref is built the compiled reference is run as well."""
     from oracle.oracle import RNG_WH, Ref, have_ref
     X, src, tgt, nt = dataset["X"], dataset["source"], dataset["target"], dataset["node_type"]
     o = oracle.mcmc(X, src, tgt, nt, max_par=3, n_iter=3000, output=10, rng_kind=RNG_WH)
     assert o.FN.max() <= 44 and o.additions[-1] > 5
+    want = np.load(os.path.join(GOLDEN, "denser_maxpar3.npz"))
+    for k in INT_COLS + ("globalLL",):
+        assert np.array_equal(getattr(o, k), want[k]), k
     if have_ref():
         r = Ref().main_fun(X, src, tgt, nt, MaxPar=3, N=3000, output=10, rng_kind=RNG_WH, seeds=(10437, 13568, 30524))
         for k in INT_COLS + ("globalLL",):

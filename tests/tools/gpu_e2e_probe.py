@@ -1,6 +1,6 @@
 import os, sys, time
 import numpy as np, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 from bayesnetworks_b200 import Context
 from bayesnetworks_b200.synth import chain_seeds, make_dag, make_prior, simulate_torch
 P, N, MP, chains, iters = 1000, 100000, 8, 64, 100000
