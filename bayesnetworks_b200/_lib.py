@@ -24,7 +24,7 @@ EXPORTED_SYMBOLS = (
     "bn_create_from_stats", "bn_block_colsum_device", "bn_block_gram_device", "bn_create_from_stats_device",
     "bn_destroy", "bn_trim_pool", "bn_set_stream", "bn_set_default_stream", "bn_get_stats", "bn_get_gram_ms",
     "bn_get_launch_count", "bn_score_nodes", "bn_score_all_proposals",
-    "bn_score_all_proposals_device", "bn_run", "bn_main_fun",
+    "bn_score_all_proposals_device", "bn_run", "bn_main_fun", "bn_score_state_len",
 )
 
 _dp = C.POINTER(C.c_double)
@@ -64,7 +64,15 @@ class RunArgs(C.Structure):
                 ("replay_len", C.c_int64), ("initial_network", C.c_int), ("drop", C.c_int),
                 ("n_iter", C.c_int), ("output_every", C.c_int), ("device_outputs", C.c_int),
                 ("moves_capacity", C.c_int), ("n_moves", _ip), ("moves", _ip), ("edge_freq", _ip),
-                ("npar_freq", _ip), ("mt_state_in", _ip), ("mt_state_out", _ip)]
+                ("npar_freq", _ip), ("mt_state_in", _ip), ("mt_state_out", _ip),
+                ("start_parents", _ip), ("start_n_par", _ip), ("state_in", C.c_void_p), ("state_out", C.c_void_p),
+                ("score_state_in", _dp), ("score_state_out", _dp)]
+
+
+class ChainStateC(C.Structure):
+    """bn_chain_state"""
+    _fields_ = [("iter", C.c_int64), ("valid", C.c_int), ("total_edges_member", C.c_int),
+                ("additions", C.c_int), ("deletions", C.c_int), ("wh_state", C.c_int * 3), ("uniforms", C.c_int64)]
 
 
 _lib = None
@@ -107,6 +115,7 @@ def lib() -> C.CDLL:
     L.bn_score_all_proposals_device.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 5 + [C.POINTER(C.c_float)]
     L.bn_run.argtypes = [C.c_void_p, C.POINTER(RunArgs), C.POINTER(Trace), C.c_void_p, C.c_void_p,
                          C.c_void_p, C.POINTER(C.c_float)]
+    L.bn_score_state_len.argtypes = [C.c_void_p, C.POINTER(C.c_int64)]
     L.bn_main_fun.argtypes = ([C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
                                C.c_void_p, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int, C.c_int,
                                C.c_int, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 10)

@@ -47,11 +47,100 @@ class ChainResult:
     npar_freq: Optional[np.ndarray] = None       # [node, k] iterations spent with k parents
     kernel_cycles: int = 0                       # SM cycles of the chain, first to last iteration
     mt_state: Optional[np.ndarray] = None        # R-MT stream state after the run (.Random.seed[2:626])
+    state: Optional["ChainState"] = None         # run(want_state=True): where the chain continues from
 
     def edges(self):
         """(parent, child) pairs, 0-based, per-child list order."""
         return [(int(self.final_parents[c, e]), c)
                 for c in range(len(self.final_npar)) for e in range(int(self.final_npar[c]))]
+
+
+_STATE_SCALARS = ("iter", "valid", "total_edges_member", "additions", "deletions", "uniforms")
+
+
+@dataclass
+class ChainState:
+    """Where a chain continues from: its ordered parent lists, the scalars of ``bn_chain_state``, its
+    uniform stream and, optionally, its score block (per-node scores, and for max_par > 8 the per-node
+    Cholesky factors).  ``Context.run(start=[...])`` continues each chain with ``n_iter`` more iterations;
+    a run split into segments this way computes the same bits as the uninterrupted run.
+
+    A state made by :meth:`from_graph` / :meth:`from_edges` is a fresh chain from that graph (iteration 0,
+    the stream from the run's seeds); ``rng`` and ``n_samples`` are then None.  A state returned by a run
+    (``ChainResult.state``) is a resume and only fits a run with the same node count, max_par, sample
+    count and stream kind."""
+    parents: np.ndarray                      # [P, max_par] int32, -1 padded, list order
+    npar: np.ndarray                         # [P] int32
+    n_samples: Optional[int] = None
+    rng: Optional[int] = None                # BN_RNG_* of the stream to continue; None = fresh start
+    iter: int = 0                            # next iteration index
+    valid: int = 1                           # the stale `valid` flag
+    total_edges_member: int = 0              # TotalEdges as the last LogPrior() left it
+    additions: int = 0                       # accepted moves since `drop` (trace columns)
+    deletions: int = 0
+    uniforms: int = 0                        # uniforms consumed since iteration 0
+    wh_state: Optional[np.ndarray] = None    # rng WH: the stream state (a seed triple)
+    mt_state: Optional[np.ndarray] = None    # rng RMT: .Random.seed[2:626] after the consumed uniforms
+    score_block: Optional[np.ndarray] = None  # float64 [Context.score_state_len]
+
+    @property
+    def P(self) -> int:
+        return int(self.npar.shape[0])
+
+    @property
+    def max_par(self) -> int:
+        return int(self.parents.shape[1])
+
+    @property
+    def resumed(self) -> bool:
+        return self.rng is not None
+
+    @classmethod
+    def from_graph(cls, parents, npar) -> "ChainState":
+        """A fresh chain from ordered parent lists ([P, max_par], -1 padded) and their lengths."""
+        parents, npar = as_i32(parents), as_i32(npar)
+        if parents.ndim != 2 or npar.shape != (parents.shape[0],):
+            raise ValueError("parents must be (P, max_par) and npar (P,)")
+        return cls(parents=parents.copy(), npar=npar.copy())
+
+    @classmethod
+    def from_edges(cls, edges, n_nodes: int, max_par: int) -> "ChainState":
+        """A fresh chain from 0-based (parent, child) pairs; each child's parents keep the pairs' order."""
+        parents = np.full((n_nodes, max_par), -1, dtype=np.int32)
+        npar = np.zeros(n_nodes, dtype=np.int32)
+        for j, c in edges:
+            if npar[c] >= max_par:
+                raise ValueError(f"node {c} has more than max_par = {max_par} parents")
+            parents[c, npar[c]] = j
+            npar[c] += 1
+        return cls(parents=parents, npar=npar)
+
+    def save(self, path) -> None:
+        """Write the state as .npz (a checkpoint that outlives the process)."""
+        d = {"parents": self.parents, "npar": self.npar}
+        for k in _STATE_SCALARS:
+            d[k] = np.int64(getattr(self, k))
+        for k in ("n_samples", "rng"):
+            if getattr(self, k) is not None:
+                d[k] = np.int64(getattr(self, k))
+        for k in ("wh_state", "mt_state", "score_block"):
+            if getattr(self, k) is not None:
+                d[k] = getattr(self, k)
+        np.savez(path, **d)
+
+    @classmethod
+    def load(cls, path) -> "ChainState":
+        with np.load(path) as z:
+            kw = {k: int(z[k]) for k in _STATE_SCALARS}
+            for k in ("n_samples", "rng"):
+                kw[k] = int(z[k]) if k in z else None
+            for k in ("wh_state", "mt_state", "score_block"):
+                kw[k] = z[k].copy() if k in z else None
+            return cls(parents=z["parents"].copy(), npar=z["npar"].copy(), **kw)
+
+
+def _bad_arg(msg):
+    return BnError(_lib.BN_ERR_BAD_ARG, msg)
 
 
 def _i32_bits(a) -> np.ndarray:
@@ -210,14 +299,71 @@ class Context:
         return float(ms.value)
 
     # -- chains --------------------------------------------------------------
+    @property
+    def score_state_len(self) -> int:
+        """Per-chain length (doubles) of ``ChainState.score_block``."""
+        n = C.c_int64(0)
+        check(_lib.lib().bn_score_state_len(self._h, C.byref(n)))
+        return int(n.value)
+
+    def _start_args(self, start, n_chains, kind, args, keep):
+        """bn_run_args.start_parents / state_in / score_state_in / mt_state_in from ChainStates."""
+        p, mp = self.n_nodes, self.max_par
+        if len(start) != n_chains:
+            raise _bad_arg(f"start holds {len(start)} states for {n_chains} chains")
+        for c, st in enumerate(start):
+            if st.P != p or st.max_par != mp:
+                raise _bad_arg(f"start state of chain {c} is for P={st.P}, max_par={st.max_par}; "
+                               f"the context has P={p}, max_par={mp}")
+            if st.resumed and (st.rng != kind or st.n_samples != self.n_samples):
+                raise _bad_arg(f"start state of chain {c} continues a stream of kind {st.rng} over "
+                               f"{st.n_samples} samples; this run is kind {kind} over {self.n_samples}")
+        resumed = {st.resumed for st in start}
+        if len(resumed) > 1:
+            raise _bad_arg("start mixes fresh and resumed chains")
+        par = np.ascontiguousarray(np.stack([as_i32(st.parents) for st in start]))
+        npar = np.ascontiguousarray(np.stack([as_i32(st.npar) for st in start]))
+        keep += [par, npar]
+        args.start_parents, args.start_n_par = par.ctypes.data_as(_lib._ip), npar.ctypes.data_as(_lib._ip)
+        if resumed.pop():
+            sts = (_lib.ChainStateC * n_chains)()
+            for c, st in enumerate(start):
+                o = sts[c]
+                for k in _STATE_SCALARS:
+                    setattr(o, k, int(getattr(st, k)))
+                if kind == BN_RNG_WH:
+                    o.wh_state[:] = [int(v) for v in st.wh_state]
+            keep.append(sts)
+            args.state_in = C.cast(sts, C.c_void_p)
+            if kind == BN_RNG_RMT:
+                mt_in = np.ascontiguousarray(np.stack([_i32_bits(st.mt_state) for st in start]))
+                keep.append(mt_in)
+                args.mt_state_in = mt_in.ctypes.data_as(_lib._ip)
+        blocks = [st.score_block is not None for st in start]
+        if any(blocks):
+            if not all(blocks):
+                raise _bad_arg("start gives a score block for some chains only")
+            sb = np.ascontiguousarray(np.stack([np.asarray(st.score_block, dtype=np.float64) for st in start]))
+            if sb.shape[1] != self.score_state_len:
+                raise _bad_arg(f"score block of {sb.shape[1]} doubles; this context needs {self.score_state_len}")
+            keep.append(sb)
+            args.score_state_in = sb.ctypes.data_as(_lib._dp)
+
     def run(self, n_chains=1, n_iter=1000, output=100, initial_network=2, drop=0, rng="wh",
             seeds=None, replay=None, log_moves=False, moves_capacity=None, tabulate=False,
-            mt_state=None, want_mt_state=False):
+            mt_state=None, want_mt_state=False, start=None, want_state=False):
         """Run ``n_chains`` independent chains; returns (list[ChainResult], kernel_ms).
 
         ``mt_state`` (rng="rmt"): R's stream state per chain, ``.Random.seed[2:626]`` (625 ints:
         position + 624 words), instead of ``set.seed(seeds)``; ``want_mt_state`` returns the
-        state after the run in ``ChainResult.mt_state``."""
+        state after the run in ``ChainResult.mt_state``.
+
+        ``start``: one :class:`ChainState` per chain.  Fresh states start the chains from their graphs
+        (``initial_network`` is not read); resumed states continue each chain for ``n_iter`` more
+        iterations with its own stream (rng="replay": ``replay`` holds the remaining uniforms, the
+        original buffer from ``state.uniforms`` on).  ``want_state`` returns the state to continue
+        from in ``ChainResult.state``, score block included.  Trace, move log and tabulation cover
+        the iterations of this call."""
         L = _lib.lib()
         kind = _RNG_KINDS[rng]
         p, mp = self.n_nodes, self.max_par
@@ -277,6 +423,21 @@ class Context:
             args.edge_freq = freq.ctypes.data_as(_lib._ip)
             nfreq = np.zeros((n_chains, p, mp + 1), dtype=np.int32)
             args.npar_freq = nfreq.ctypes.data_as(_lib._ip)
+        keep = []
+        if start is not None:
+            self._start_args(start, n_chains, kind, args, keep)
+            if kind == BN_RNG_RMT and start[0].resumed and mt_out is None:
+                mt_out = np.zeros((n_chains, 625), dtype=np.int32)
+                args.mt_state_out = mt_out.ctypes.data_as(_lib._ip)
+        st_out = sb_out = None
+        if want_state:
+            st_out = (_lib.ChainStateC * n_chains)()
+            args.state_out = C.cast(st_out, C.c_void_p)
+            sb_out = np.empty((n_chains, self.score_state_len))
+            args.score_state_out = sb_out.ctypes.data_as(_lib._dp)
+            if kind == BN_RNG_RMT and mt_out is None:
+                mt_out = np.zeros((n_chains, 625), dtype=np.int32)
+                args.mt_state_out = mt_out.ctypes.data_as(_lib._ip)
         fpar = np.empty((n_chains, p, mp), dtype=np.int32)   # the library pads unused slots with -1
         fnpar = np.empty((n_chains, p), dtype=np.int32)
         stats = (_lib.ChainStats * n_chains)()
@@ -306,6 +467,13 @@ class Context:
                 accepted_moves=None if moves is None else moves[ch, :int(n_moves[ch])],
                 edge_freq=None if freq is None else freq[ch],
                 npar_freq=None if nfreq is None else nfreq[ch]))
+            if st_out is not None:
+                o = st_out[ch]
+                out[-1].state = ChainState(
+                    parents=fpar[ch].copy(), npar=fnpar[ch].copy(), n_samples=self.n_samples, rng=kind,
+                    wh_state=np.array(o.wh_state[:], dtype=np.int32) if kind == BN_RNG_WH else None,
+                    mt_state=mt_out[ch].copy() if kind == BN_RNG_RMT else None, score_block=sb_out[ch],
+                    **{k: int(getattr(o, k)) for k in _STATE_SCALARS})
         return out, float(ms.value)
 
 

@@ -6,6 +6,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -664,31 +665,59 @@ static void rmt_seed_state(uint32_t seed, uint32_t* mt) {
   }
 }
 
-// R's MT_genrand state step (R sources, src/main/RNG.c): advance (mt, mti) by n_draws uniforms.
-// Bookkeeping of the stream position for mt_state_out only -- the uniforms themselves are
-// generated on the device (rng_core.cuh).
-static void rmt_advance(uint32_t* mt, int& mti, int64_t n_draws) {
-  const int N = 624, M = 397;
-  const uint32_t UPPER = 0x80000000u, LOWER = 0x7fffffffu, MAG = 0x9908b0dfu;
-  while (n_draws > 0) {
-    if (mti >= N) {
-      int kk = 0;
-      for (; kk < N - M; kk++) {
-        const uint32_t y = (mt[kk] & UPPER) | (mt[kk + 1] & LOWER);
-        mt[kk] = mt[kk + M] ^ (y >> 1) ^ ((y & 1u) ? MAG : 0u);
+// Supplied start graphs (bn_run_args.start_parents): lists in range, -1 padded, without self-loops or
+// duplicates, and acyclic (the ancestor bitsets of the chain assume a DAG).
+static int check_start_graphs(int nc, int P, int MP, const int* par, const int* npar) {
+  std::vector<int> indeg(P), order, kids_n(P), kids_off(P + 1), kids;
+  for (int ch = 0; ch < nc; ch++) {
+    const int* pc = par + (size_t)ch * P * MP;
+    const int* nc_ = npar + (size_t)ch * P;
+    std::fill(kids_n.begin(), kids_n.end(), 0);
+    for (int c = 0; c < P; c++) {
+      const int k = nc_[c];
+      if (k < 0 || k > MP) return fail(BN_ERR_BAD_ARG, "start graph of chain %d: node %d has %d parents (max_par = %d)", ch, c, k, MP);
+      for (int e = 0; e < MP; e++) {
+        const int q = pc[(size_t)c * MP + e];
+        if (e >= k) {
+          if (q != -1) return fail(BN_ERR_BAD_ARG, "start graph of chain %d: node %d, slot %d beyond its %d parents is not -1", ch, c, e, k);
+          continue;
+        }
+        if (q < 0 || q >= P) return fail(BN_ERR_BAD_ARG, "start graph of chain %d: node %d has parent %d out of range", ch, c, q);
+        if (q == c) return fail(BN_ERR_BAD_ARG, "start graph of chain %d: node %d is its own parent", ch, c);
+        for (int f = 0; f < e; f++)
+          if (pc[(size_t)c * MP + f] == q) return fail(BN_ERR_BAD_ARG, "start graph of chain %d: node %d lists parent %d twice", ch, c, q);
+        kids_n[q]++;
       }
-      for (; kk < N - 1; kk++) {
-        const uint32_t y = (mt[kk] & UPPER) | (mt[kk + 1] & LOWER);
-        mt[kk] = mt[kk + (M - N)] ^ (y >> 1) ^ ((y & 1u) ? MAG : 0u);
-      }
-      const uint32_t y = (mt[N - 1] & UPPER) | (mt[0] & LOWER);
-      mt[N - 1] = mt[M - 1] ^ (y >> 1) ^ ((y & 1u) ? MAG : 0u);
-      mti = 0;
     }
-    const int64_t take = n_draws < (int64_t)(N - mti) ? n_draws : (int64_t)(N - mti);
-    mti += (int)take;
-    n_draws -= take;
+    // Kahn: every node must come off the queue
+    kids_off[0] = 0;
+    for (int c = 0; c < P; c++) kids_off[c + 1] = kids_off[c] + kids_n[c];
+    kids.assign(kids_off[P], 0);
+    std::fill(kids_n.begin(), kids_n.end(), 0);
+    order.clear();
+    for (int c = 0; c < P; c++) {
+      indeg[c] = nc_[c];
+      if (!indeg[c]) order.push_back(c);
+      for (int e = 0; e < nc_[c]; e++) { const int q = pc[(size_t)c * MP + e]; kids[kids_off[q] + kids_n[q]++] = c; }
+    }
+    for (size_t i = 0; i < order.size(); i++)
+      for (int t = kids_off[order[i]]; t < kids_off[order[i] + 1]; t++)
+        if (--indeg[kids[t]] == 0) order.push_back(kids[t]);
+    if ((int)order.size() < P)
+      for (int c = 0; c < P; c++)
+        if (indeg[c] > 0) return fail(BN_ERR_BAD_ARG, "start graph of chain %d is cyclic: node %d lies on or behind a cycle", ch, c);
   }
+  return BN_OK;
+}
+
+static int64_t score_state_len(int P, int MP) {
+  return (int64_t)P + (MP > 8 ? (int64_t)P * fac_stride(fac_mp(MP)) : 0);
+}
+
+extern "C" int bn_score_state_len(bn_ctx* c, int64_t* n) {
+  if (!c || !n) return fail(BN_ERR_BAD_ARG, "NULL argument");
+  *n = score_state_len(c->P, c->max_par);
+  return BN_OK;
 }
 
 struct DevBuf {  // frees on scope exit
@@ -723,9 +752,29 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
   if (!trace->n_rows || !trace->iter || !trace->changed_node || !trace->movetype || !trace->global_ll ||
       !trace->additions || !trace->deletions || !trace->fn || !trace->fp)
     return fail(BN_ERR_BAD_ARG, "trace column pointer is NULL");
+  // supplied start graphs and resumed chains
+  const bool given = a->start_parents != nullptr, resume = a->state_in != nullptr;
+  const bool with_state = given || a->state_out || a->score_state_out;
+  if ((resume || a->score_state_in) && !given) return fail(BN_ERR_BAD_ARG, "state_in / score_state_in need start_parents");
+  if (given && !a->start_n_par) return fail(BN_ERR_BAD_ARG, "start_parents needs start_n_par");
+  if (resume && a->rng_kind == BN_RNG_RMT && !a->mt_state_in)
+    return fail(BN_ERR_BAD_ARG, "resuming an R Mersenne-Twister stream needs mt_state_in");
+  if (given) {
+    const int rc = check_start_graphs(nc, c->P, c->max_par, a->start_parents, a->start_n_par);
+    if (rc) return rc;
+  }
+  if (resume)
+    for (int ch = 0; ch < nc; ch++) {
+      const bn_chain_state& st = a->state_in[ch];
+      if (st.iter < 0 || st.iter + a->n_iter > 0x7fffffffll)
+        return fail(BN_ERR_BAD_ARG, "state_in of chain %d: iteration %lld + n_iter %d is outside 0..INT_MAX", ch,
+                    (long long)st.iter, a->n_iter);
+      if (st.valid != 0 && st.valid != 1) return fail(BN_ERR_BAD_ARG, "state_in of chain %d: valid = %d (0 or 1)", ch, st.valid);
+    }
   CU_TRY(cudaSetDevice(c->device));
 
   const int64_t P = c->P, MP = c->max_par, W = (P + 31) / 32;
+  const int64_t slen = score_state_len((int)P, (int)MP);
   const int64_t cap = trace->capacity > 0 ? trace->capacity : 1;
   StageTimer tm("bn_run");
   DevBuf buf;
@@ -744,7 +793,7 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
     q.P = (int)P; q.max_par = (int)MP; q.W = (int)W;
     // (its team operations are dealt over the seven helper warps: larger row lists per part)
     const int sn = scratch_words((int)P, HELPER_WARPS, 32) > w.scratch_n ? scratch_words((int)P, HELPER_WARPS, 32) : w.scratch_n;
-    w.pipeline = (e && e[0] != '0' && MP <= 8 && 2 * nc <= n_sm && chains_can_pipeline(q, sn)) ? 1 : 0;
+    w.pipeline = (e && e[0] != '0' && !with_state && MP <= 8 && 2 * nc <= n_sm && chains_can_pipeline(q, sn)) ? 1 : 0;
     if (w.pipeline) w.scratch_n = sn;
     if (w.pipeline && e && (e[0] == '3' || e[0] == '5')) w.pipeline = e[0] - '0';  // (developer switch: the chain's CTA rebuilds every window itself)
   }
@@ -764,6 +813,37 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
   }
   CU_TRY(cudaMemsetAsync(w.dscore, 0xff, dscore_n * sizeof(double), c->stream));  // NaN = unknown (tags: -1)
   const bool dev_out = a->device_outputs != 0;
+  if (given) {
+    int *d_sp = nullptr, *d_sn = nullptr;
+    CU_TRY(buf.alloc(&d_sp, (size_t)(nc * P * MP)));
+    CU_TRY(buf.alloc(&d_sn, (size_t)(nc * P)));
+    CU_TRY(cudaMemcpyAsync(d_sp, a->start_parents, (size_t)(nc * P * MP) * 4, cudaMemcpyHostToDevice, c->stream));
+    CU_TRY(cudaMemcpyAsync(d_sn, a->start_n_par, (size_t)(nc * P) * 4, cudaMemcpyHostToDevice, c->stream));
+    w.start_par = d_sp; w.start_npar = d_sn;
+  }
+  std::vector<ChainStart> starts;
+  if (resume) {
+    starts.resize(nc);
+    for (int ch = 0; ch < nc; ch++) {
+      const bn_chain_state& st = a->state_in[ch];
+      starts[ch].iter = st.iter; starts[ch].valid = st.valid; starts[ch].te_m = st.total_edges_member;
+      starts[ch].acc_add = st.additions; starts[ch].acc_del = st.deletions;
+    }
+    ChainStart* d_st = nullptr;
+    CU_TRY(buf.alloc(&d_st, (size_t)nc));
+    CU_TRY(cudaMemcpyAsync(d_st, starts.data(), sizeof(ChainStart) * nc, cudaMemcpyHostToDevice, c->stream));
+    w.start = d_st;
+  }
+  // score block [base P | factors P x fac_stride] per chain <-> w.base, w.fac
+  const cudaMemcpyKind sc_in = dev_out ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+  if (a->score_state_in) {
+    CU_TRY(cudaMemcpy2DAsync(w.base, P * 8, a->score_state_in, slen * 8, P * 8, nc, sc_in, c->stream));
+    if (MP > 8)
+      CU_TRY(cudaMemcpy2DAsync(w.fac, (slen - P) * 8, a->score_state_in + P, slen * 8, (slen - P) * 8, nc, sc_in, c->stream));
+    w.scores_in = 1;
+  }
+  w.scores_out = a->score_state_out ? 1 : 0;
+  w.with_state = with_state || a->state_in || a->score_state_in;
   if (dev_out) {
     w.t_iter = trace->iter; w.t_changed = trace->changed_node; w.t_movetype = trace->movetype;
     w.t_gll = trace->global_ll; w.t_add = trace->additions; w.t_del = trace->deletions;
@@ -809,6 +889,8 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
       }
     }
   }
+  if (resume && a->rng_kind == BN_RNG_WH)  // the stream continues from the state the stopped run returned
+    for (int ch = 0; ch < nc; ch++) memcpy(&seeds[3 * ch], a->state_in[ch].wh_state, 3 * sizeof(int));
   if (a->rng_kind == BN_RNG_WH) {
     for (int ch = 0; ch < nc; ch++) {
       const int* s = &seeds[3 * ch];
@@ -923,6 +1005,19 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
       out[0] = pos;
       for (int i = 0; i < 624; i++) out[1 + i] = (int)st[i];
     }
+    if (a->state_out) {
+      bn_chain_state& o = a->state_out[ch];
+      memset(&o, 0, sizeof(o));
+      o.iter = res[ch].end.iter; o.valid = res[ch].end.valid; o.total_edges_member = res[ch].end.te_m;
+      o.additions = res[ch].end.acc_add; o.deletions = res[ch].end.acc_del;
+      o.uniforms = (resume ? a->state_in[ch].uniforms : 0) + res[ch].uniforms;
+      if (a->rng_kind == BN_RNG_WH) wh_advance(&seeds[3 * ch], res[ch].uniforms, o.wh_state);
+    }
+  }
+  if (a->score_state_out) {
+    const cudaMemcpyKind k = dev_out ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    CU_TRY(cudaMemcpy2D(a->score_state_out, slen * 8, w.base, P * 8, P * 8, nc, k));
+    if (MP > 8) CU_TRY(cudaMemcpy2D(a->score_state_out + P, slen * 8, w.fac, (slen - P) * 8, (slen - P) * 8, nc, k));
   }
   const cudaMemcpyKind out_kind = dev_out ? cudaMemcpyHostToDevice : cudaMemcpyHostToHost;
   CU_TRY(cudaMemcpy(trace->n_rows, nrows.data(), (size_t)nc * 4, out_kind));

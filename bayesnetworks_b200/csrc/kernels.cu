@@ -21,7 +21,11 @@ namespace bn {
 // ALL_SMEM: every per-chain array of the plan sits in dynamic shared memory, so the pointers
 // have a provable shared-memory provenance and the state accesses compile to LDS/STS
 // instead of generic loads.
-template <int KMAX, bool ALL_SMEM>
+// WITH_STATE: the chains start from supplied graphs / resume states or export their state
+// (ChainWorkspace.with_state).  Without it the start pointers stay null at compile time, so chain_init
+// folds to the start of initial_network and the steady-state loop compiles as it did before resumable
+// chains existed (a per-chain end iteration would hold a register for the whole loop).
+template <int KMAX, bool ALL_SMEM, bool WITH_STATE>
 __global__ void __launch_bounds__((HELPER_WARPS + 1) * 32, 1) chain_kernel(ChainParams p, ChainWorkspace w, ChainRngArgs ra,
                                                    ChainSmemPlan sm, ChainResult* __restrict__ results) {
   __shared__ double ubuf[RNG_CAP];
@@ -67,6 +71,11 @@ __global__ void __launch_bounds__((HELPER_WARPS + 1) * 32, 1) chain_kernel(Chain
   m.fac = w.fac ? w.fac + ch * P * fac_stride(fac_mp(p.max_par)) : nullptr;   // (MaxPar > 8 only)
   m.rowbuf = w.rowbuf ? w.rowbuf + (int64_t)ch * REPLAY_POS * row_stride(fac_mp(p.max_par)) : nullptr;
   m.helper = helper_cmd;
+  if constexpr (WITH_STATE) {
+    if (w.start_par) { m.start_par = w.start_par + ch * P * MP; m.start_npar = w.start_npar + ch * P; }
+    if (w.start) m.start = w.start + ch;
+    if (w.scores_in) m.base_in = w.base + ch * P;
+  }
 
   RngStream rng;
   if (ra.kind == RNG_WH)
@@ -84,6 +93,8 @@ __global__ void __launch_bounds__((HELPER_WARPS + 1) * 32, 1) chain_kernel(Chain
   pp.sc.half_n = (double)p.n_samples / 2.0;
   pp.sc.ratio = dof_ratio;
   if (!m.moves) pp.moves_capacity = 0;
+  if constexpr (WITH_STATE)
+    if (w.start) pp.n_iter = (int)(w.start[ch].iter + p.n_iter);  // the chain ends n_iter iterations after its start
   if (ALL_SMEM || sm.off_types >= 0) {
     uint8_t* t = (uint8_t*)(dyn_smem + sm.off_types);
     for (int i = threadIdx.x; i < p.P; i += blockDim.x) t[i] = p.node_type[i];
@@ -107,9 +118,16 @@ __global__ void __launch_bounds__((HELPER_WARPS + 1) * 32, 1) chain_kernel(Chain
     for (int64_t i = lane; i < P * MP; i += 32) g_par[i] = m.par[i];
   if (ALL_SMEM || sm.off_npar >= 0)
     for (int64_t i = lane; i < P; i += 32) g_npar[i] = m.npar[i];
+  if constexpr (WITH_STATE)
+    if (w.scores_out && (ALL_SMEM || sm.off_base >= 0))
+      for (int64_t i = lane; i < P; i += 32) w.base[ch * P + i] = m.base[i];
 
   if (lane == 0) {
     ChainResult& r = results[ch];
+    if constexpr (WITH_STATE) {
+      r.end.iter = s.iter; r.end.valid = s.valid; r.end.te_m = s.te_m;
+      r.end.acc_add = s.acc_add; r.end.acc_del = s.acc_del;
+    }
     r.uniforms = s.read_pos;
     r.valid_iters = s.valid_iters;
     r.alg_bytes = s.alg_bytes;
@@ -368,7 +386,7 @@ static const char* launch_chains_t(ChainParams p, const ChainWorkspace& w, const
     if (w.pipeline) return "two-CTA chains requested but the state does not fit in shared memory";
   }
   cudaFuncAttributes fa;
-  if (cudaFuncGetAttributes(&fa, chain_kernel<KMAX, true>) != cudaSuccess) return "cudaFuncGetAttributes failed";
+  if (cudaFuncGetAttributes(&fa, chain_kernel<KMAX, true, false>) != cudaSuccess) return "cudaFuncGetAttributes failed";
   int dev = 0, max_optin = 0;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
@@ -376,7 +394,8 @@ static const char* launch_chains_t(ChainParams p, const ChainWorkspace& w, const
   ChainSmemPlan sm = plan_chain_smem(p, w.scratch_n, budget > 0 ? budget : 0);
   const bool all_smem = sm.off_types >= 0 && sm.off_npar >= 0 && sm.off_base >= 0 && sm.off_haspar >= 0 &&
                         sm.off_hplist >= 0 && sm.off_par >= 0 && sm.off_scratch >= 0 && sm.off_anc >= 0;
-  auto kernel = all_smem ? chain_kernel<KMAX, true> : chain_kernel<KMAX, false>;
+  auto kernel = w.with_state ? (all_smem ? chain_kernel<KMAX, true, true> : chain_kernel<KMAX, false, true>)
+                             : (all_smem ? chain_kernel<KMAX, true, false> : chain_kernel<KMAX, false, false>);
   if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, sm.total_bytes) != cudaSuccess)
     return "cudaFuncSetAttribute(chain_kernel) failed";
   if (getenv("BN_B200_CLUSTER_EXPERIMENT") && n_chains % 2 == 0) {

@@ -20,6 +20,12 @@ struct ChainWorkspace {  // arrays over all chains of a run (device memory)
   double* rowbuf;                      // [nc][REPLAY_POS][row_stride(max_par)] candidate rows of a round
   int pipeline;                        // 1: two CTAs per chain (chain_pipe_kernel): dscore holds (score, tag) pairs,
                                        // the R-MT states are [2][nc][624] (one copy per CTA)
+  // supplied starts (one-CTA kernel only; null = the start graph of initial_network)
+  const int* start_par; const int* start_npar;  // [nc][P][max_par], [nc][P]
+  const ChainStart* start;             // [nc] resumed chains: each runs n_iter iterations from its start->iter
+  int scores_in;                       // base (and fac) already hold the chains' scores and factors
+  int scores_out;                      // write the final scores back to base when they lived in shared memory
+  int with_state;                      // any of the above, or the chains' end state wanted: the WITH_STATE kernels
 };
 
 // Which per-chain arrays live in dynamic shared memory (byte offset, -1 = global memory).
@@ -50,6 +56,7 @@ struct ChainResult {
   long long cyc[12], slots_sim, cyc_total;
   long long pipe_cyc[6];
   int pipe[4];  // two-CTA form: windows requested, waits for the builder, windows discarded, in-place rebuilds
+  ChainStart end;  // (one-CTA kernel) the scalars to resume from
 };
 
 struct SweepParams {

@@ -148,4 +148,48 @@ BN_HD void rng_top_up(RngStream& r, int64_t read_pos) {
   while (r.gen_hi + Warp::NL <= read_pos + RNG_CAP) rng_fill_chunk(r);
 }
 
+// ---- host bookkeeping of a stream's position (the uniforms themselves come from the device) ----
+
+// Wichmann-Hill state after n_draws uniforms from (ix, iy, iz): x a^n mod m per LCG, itself a valid
+// seed triple.  A state that reduces to 0 is written as the modulus (the same residue, and a seed the
+// range check accepts).
+inline void wh_advance(const int* in, int64_t n_draws, int* out) {
+  const uint64_t a[3] = {171u, 172u, 170u}, mod[3] = {30269u, 30307u, 30323u};
+  for (int t = 0; t < 3; t++) {
+    if (n_draws == 0) { out[t] = in[t]; continue; }
+    uint64_t r = 1, b = a[t];
+    for (int64_t e = n_draws; e > 0; e >>= 1) {
+      if (e & 1) r = r * b % mod[t];
+      b = b * b % mod[t];
+    }
+    r = r * (uint64_t)in[t] % mod[t];
+    out[t] = r == 0 ? (int)mod[t] : (int)r;
+  }
+}
+
+// R's MT_genrand state step (R sources, src/main/RNG.c): advance (mt, mti) by n_draws uniforms.
+inline void rmt_advance(uint32_t* mt, int& mti, int64_t n_draws) {
+  const int N = 624, M = 397;
+  const uint32_t UPPER = 0x80000000u, LOWER = 0x7fffffffu, MAG = 0x9908b0dfu;
+  while (n_draws > 0) {
+    if (mti >= N) {
+      int kk = 0;
+      for (; kk < N - M; kk++) {
+        const uint32_t y = (mt[kk] & UPPER) | (mt[kk + 1] & LOWER);
+        mt[kk] = mt[kk + M] ^ (y >> 1) ^ ((y & 1u) ? MAG : 0u);
+      }
+      for (; kk < N - 1; kk++) {
+        const uint32_t y = (mt[kk] & UPPER) | (mt[kk + 1] & LOWER);
+        mt[kk] = mt[kk + (M - N)] ^ (y >> 1) ^ ((y & 1u) ? MAG : 0u);
+      }
+      const uint32_t y = (mt[N - 1] & UPPER) | (mt[0] & LOWER);
+      mt[N - 1] = mt[M - 1] ^ (y >> 1) ^ ((y & 1u) ? MAG : 0u);
+      mti = 0;
+    }
+    const int64_t take = n_draws < (int64_t)(N - mti) ? n_draws : (int64_t)(N - mti);
+    mti += (int)take;
+    n_draws -= take;
+  }
+}
+
 }  // namespace bn

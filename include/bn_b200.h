@@ -198,6 +198,17 @@ typedef struct bn_chain_stats {
                               phase_cycles are filled by diagnostics builds only (-DBN_PHASE_CYCLES) */
 } bn_chain_stats;
 
+/* What a chain carries across a segment boundary besides its graph, its scores and its stream. */
+typedef struct bn_chain_state {
+  int64_t iter;              /* next iteration index */
+  int valid;                 /* the stale `valid` flag, src/bayesnet_mcmc.cpp:40 (0 or 1) */
+  int total_edges_member;    /* TotalEdges as the last LogPrior() left it, src/network.h:262-267 */
+  int additions, deletions;  /* accepted moves since `drop` (trace columns) */
+  int wh_state[3];           /* BN_RNG_WH: the stream state, a seed triple (state_out: after the uniforms
+                                consumed); 0 for the other streams */
+  int64_t uniforms;          /* uniforms consumed since iteration 0 (random start graph included) */
+} bn_chain_state;
+
 typedef struct bn_run_args {
   int n_chains;
   int rng_kind;            /* BN_RNG_* */
@@ -236,7 +247,40 @@ typedef struct bn_run_args {
      (src/RcppExports.cpp:13, src/bayesnet_mcmc.cpp:48, src/network.h:284,292,309,318,319,335). */
   const int* mt_state_in;
   int* mt_state_out;
+  /* ---- resumable chains (all NULL = the chains start as above; bn_score_state_len marks a library that has them) ----
+     A run of N iterations split into segments, each started from what the previous one returned
+     (state_out, final_parents/final_n_par, score_state_out, and the stream: wh_state, mt_state_out, or the
+     rest of the replay buffer), computes the same bits as one run of N iterations: trace, move log,
+     summed tabulations, final graph, stream state.
+     start_parents / start_n_par: [n_chains][P][max_par] (-1 padded, list order) and [n_chains][P]; HOST
+       memory.  The chains start from these graphs instead of the one initial_network names.  Each graph
+       must be acyclic, without self-loops or duplicate parents, with n_par <= max_par.
+       Without state_in this is a fresh chain from that graph: iteration 0, valid = 1, member TotalEdges 0,
+       streams from seeds / mt_state_in as above.
+     state_in: [n_chains], HOST memory, needs start_parents: a resume.  Each chain runs n_iter more
+       iterations, from state_in[c].iter up to state_in[c].iter + n_iter (<= INT_MAX).  Its stream:
+       BN_RNG_WH from wh_state (seeds are not read), BN_RNG_RMT from mt_state_in (required), BN_RNG_REPLAY
+       from `replay`, which then holds the remaining uniforms (the run's buffer from state_in[c].uniforms on).
+     state_out: [n_chains], HOST memory: the state to continue from (the graph is final_parents/final_n_par).
+     score_state_in / score_state_out: [n_chains][bn_score_state_len] doubles, host or device memory as
+       device_outputs says (score_state_in needs start_parents).  The per-node scores, followed for
+       max_par > 8 by the per-node Cholesky factors.  Without score_state_in the chains recompute them
+       from the start graphs: exactly the same bits for max_par <= 8; for max_par > 8 a factor that
+       followed accepted deletions (Givens downdates) is refactorised, which agrees to rounding only, so
+       globalLL may differ in the last bits and, very rarely, a decision with it.
+     The edge and parent-count tabulations count the iterations of this call only (from
+     max(drop, iter)); the segments' tabulations add up to the whole run's.  The opt-in two-CTA form
+     (BN_B200_PIPE) is not used when any of these fields is set: the one-CTA kernel runs instead. */
+  const int* start_parents;
+  const int* start_n_par;
+  const bn_chain_state* state_in;
+  bn_chain_state* state_out;
+  const double* score_state_in;
+  double* score_state_out;
 } bn_run_args;
+
+/* Per-chain length (doubles) of score_state_in / score_state_out. */
+int bn_score_state_len(bn_ctx* ctx, int64_t* n_doubles);
 
 /* final_parents: [n_chains][P][max_par] (-1 padded), final_n_par: [n_chains][P]; may be NULL.
  * stats: [n_chains]; may be NULL.  *kernel_ms (may be NULL) = device time of the run. */
