@@ -66,7 +66,7 @@ class RunArgs(C.Structure):
                 ("moves_capacity", C.c_int), ("n_moves", _ip), ("moves", _ip), ("edge_freq", _ip),
                 ("npar_freq", _ip), ("mt_state_in", _ip), ("mt_state_out", _ip),
                 ("start_parents", _ip), ("start_n_par", _ip), ("state_in", C.c_void_p), ("state_out", C.c_void_p),
-                ("score_state_in", _dp), ("score_state_out", _dp)]
+                ("score_state_in", _dp), ("score_state_out", _dp), ("anc_freq", _ip)]
 
 
 class ChainStateC(C.Structure):

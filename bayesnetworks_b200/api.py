@@ -48,6 +48,7 @@ class ChainResult:
     kernel_cycles: int = 0                       # SM cycles of the chain, first to last iteration
     mt_state: Optional[np.ndarray] = None        # R-MT stream state after the run (.Random.seed[2:626])
     state: Optional["ChainState"] = None         # run(want_state=True): where the chain continues from
+    anc_freq: Optional[np.ndarray] = None        # [descendant, ancestor] counts of directed paths (tabulate_ancestors)
 
     def edges(self):
         """(parent, child) pairs, 0-based, per-child list order."""
@@ -351,7 +352,7 @@ class Context:
 
     def run(self, n_chains=1, n_iter=1000, output=100, initial_network=2, drop=0, rng="wh",
             seeds=None, replay=None, log_moves=False, moves_capacity=None, tabulate=False,
-            mt_state=None, want_mt_state=False, start=None, want_state=False):
+            mt_state=None, want_mt_state=False, start=None, want_state=False, tabulate_ancestors=False):
         """Run ``n_chains`` independent chains; returns (list[ChainResult], kernel_ms).
 
         ``mt_state`` (rng="rmt"): R's stream state per chain, ``.Random.seed[2:626]`` (625 ints:
@@ -363,7 +364,12 @@ class Context:
         iterations with its own stream (rng="replay": ``replay`` holds the remaining uniforms, the
         original buffer from ``state.uniforms`` on).  ``want_state`` returns the state to continue
         from in ``ChainResult.state``, score block included.  Trace, move log and tabulation cover
-        the iterations of this call."""
+        the iterations of this call.
+
+        ``tabulate_ancestors``: ``ChainResult.anc_freq`` [descendant, ancestor] counts the tabulated
+        iterations (those ``tabulate`` counts) after which the graph has a directed path ancestor -> ... ->
+        descendant; its diagonal is the number of tabulated iterations.  Every other output is the same as
+        without it.  ``summary.ancestor_posterior`` pools chains into probabilities."""
         L = _lib.lib()
         kind = _RNG_KINDS[rng]
         p, mp = self.n_nodes, self.max_par
@@ -423,6 +429,10 @@ class Context:
             args.edge_freq = freq.ctypes.data_as(_lib._ip)
             nfreq = np.zeros((n_chains, p, mp + 1), dtype=np.int32)
             args.npar_freq = nfreq.ctypes.data_as(_lib._ip)
+        afreq = None
+        if tabulate_ancestors:
+            afreq = np.zeros((n_chains, p, p), dtype=np.int32)
+            args.anc_freq = afreq.ctypes.data_as(_lib._ip)
         keep = []
         if start is not None:
             self._start_args(start, n_chains, kind, args, keep)
@@ -466,7 +476,8 @@ class Context:
                 final_npar=fnpar[ch],
                 accepted_moves=None if moves is None else moves[ch, :int(n_moves[ch])],
                 edge_freq=None if freq is None else freq[ch],
-                npar_freq=None if nfreq is None else nfreq[ch]))
+                npar_freq=None if nfreq is None else nfreq[ch],
+                anc_freq=None if afreq is None else afreq[ch]))
             if st_out is not None:
                 o = st_out[ch]
                 out[-1].state = ChainState(

@@ -754,7 +754,8 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
     return fail(BN_ERR_BAD_ARG, "trace column pointer is NULL");
   // supplied start graphs and resumed chains
   const bool given = a->start_parents != nullptr, resume = a->state_in != nullptr;
-  const bool with_state = given || a->state_out || a->score_state_out;
+  // (the ancestor tabulation is compiled into the same kernels only: the default ones stay as they are)
+  const bool with_state = given || a->state_out || a->score_state_out || a->anc_freq;
   if ((resume || a->score_state_in) && !given) return fail(BN_ERR_BAD_ARG, "state_in / score_state_in need start_parents");
   if (given && !a->start_n_par) return fail(BN_ERR_BAD_ARG, "start_parents needs start_n_par");
   if (resume && a->rng_kind == BN_RNG_RMT && !a->mt_state_in)
@@ -863,6 +864,11 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
     if (dev_out) w.edge_freq = a->edge_freq;
     else CU_TRY(buf.alloc(&w.edge_freq, (size_t)(nc * P * P)));
     CU_TRY(cudaMemsetAsync(w.edge_freq, 0, (size_t)(nc * P * P) * 4, c->stream));
+  }
+  if (a->anc_freq) {
+    if (dev_out) w.anc_freq = a->anc_freq;
+    else CU_TRY(buf.alloc(&w.anc_freq, (size_t)(nc * P * P)));
+    CU_TRY(cudaMemsetAsync(w.anc_freq, 0, (size_t)(nc * P * P) * 4, c->stream));
   }
   if (a->npar_freq) {
     if (dev_out) w.npar_freq = a->npar_freq;
@@ -1034,6 +1040,7 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
     CU_TRY(cudaMemcpy(trace->fp, w.t_fp, n * 4, cudaMemcpyDeviceToHost));
     if (mcap) CU_TRY(cudaMemcpy(a->moves, w.moves, (size_t)nc * mcap * 16, cudaMemcpyDeviceToHost));
     if (a->edge_freq) CU_TRY(cudaMemcpy(a->edge_freq, w.edge_freq, (size_t)(nc * P * P) * 4, cudaMemcpyDeviceToHost));
+    if (a->anc_freq) CU_TRY(cudaMemcpy(a->anc_freq, w.anc_freq, (size_t)(nc * P * P) * 4, cudaMemcpyDeviceToHost));
     if (a->npar_freq) CU_TRY(cudaMemcpy(a->npar_freq, w.npar_freq, (size_t)(nc * P * (MP + 1)) * 4, cudaMemcpyDeviceToHost));
   }
   const cudaMemcpyKind fin_kind = dev_out ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;

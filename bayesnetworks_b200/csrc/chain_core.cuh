@@ -126,6 +126,8 @@ struct ChainMem {  // per-chain global memory
   const int* start_npar = nullptr;    // [P]
   const ChainStart* start = nullptr;  // a resumed chain's scalars (null: iteration 0 of a fresh chain)
   const double* base_in = nullptr;    // [P] scores to start from; with it fac already holds the factors (MaxPar > 8)
+  // posterior ancestor tabulation (anc_tab_*; null: off)
+  int* anc_freq = nullptr;            // [ancestor + descendant*P] iterations with a directed path ancestor -> descendant
 };
 
 struct ChainScalars {  // lives in registers (warp-uniform)
@@ -786,6 +788,109 @@ BN_HD void anc_after_delete(const ChainParams& p, ChainMem& m, int c, int& m_anc
 #endif
 }
 
+// ---------------------------------------------------------------------------
+// Posterior ancestor tabulation (ChainMem.anc_freq): anc_freq[a + d*P] counts the iterations, from
+// max(drop, iter) on, after which the graph has a directed path a -> ... -> d, i.e. bit a of row d.
+// No birth iteration per bit: the count is accumulated with signs.  A bit that turns on at
+// iteration t subtracts max(t, drop), one that turns off adds it, and the end of the run adds
+// max(end, drop) for every bit still set.  Only accepted moves flip bits (apply_move_vals), and they
+// flip only these, in the rows of {c} u desc(c) (the rows holding bit c; desc(c) does not change):
+//   addition j -> c   gain N & ~row, N = anc(j) & ~anc(c), read before the update (anc_tab_add)
+//   deletion at c     lose L & ~row, L = old anc(c) & ~new anc(c), read after it (anc_tab_del)
+// Lanes take (row, chunk) pairs; distinct lanes own distinct counters, so no atomics are needed.
+// ---------------------------------------------------------------------------
+// v added for every set bit of every row (chain start: -max(drop, iter); end: max(end, drop))
+BN_HD void anc_tab_all(const ChainParams& p, const ChainMem& m, int v) {
+  const int l = Warp::lane(), P = p.P, W = p.W;
+  for (int64_t i = l; i < (int64_t)P * W; i += Warp::NL) {
+    const int d = (int)(i / W), w = (int)(i - (int64_t)d * W);
+    int* out = m.anc_freq + (int64_t)d * P + 32 * w;
+    for (uint32_t b = m.anc[(int64_t)d * p.Ws + w]; b; b &= b - 1u) out[ffs32(b) - 1] += v;
+  }
+  Warp::sync();
+}
+
+// the lost / gained sets live where anc_after_delete keeps L: the chunks lay.L[lay.nzc[1..nnz]]
+BN_HD DelLayout anc_tab_layout(const ChainParams& p, const ChainMem& m) {
+  int nparts = 1;
+#if defined(__CUDA_ARCH__)
+  if (m.helper) nparts = m.pipe ? HELPER_WARPS : HELPER_WARPS + 1;
+#endif
+  return del_layout(p, m, nparts);
+}
+
+// v added at (bit a, row d) for every row d holding bit c and every bit a of L & ~row d, L = the chunks
+// L4[nzc[1..nnz]].  The rows are first listed (`rows`: lay.lists, free outside the team operations), then
+// lanes take (listed row, 32-bit word of a non-zero chunk) pairs, so that one row with many flipped bits (a
+// sink gaining a long ancestry) is still spread over lanes.  A lane reads up to eight of its counters before
+// it writes them back: the loads are independent and overlap instead of paying a memory round trip per bit.
+// Not inlined: its registers (the eight counters in flight) would otherwise raise the register pressure of
+// the whole chain loop of the WITH_STATE kernels, which resumable runs without the tabulation share.
+BN_NOINLINE void anc_tab_flip(const uint32_t* anc, int Ws, int P, int* anc_freq, int c, const uint32_t* Lw,
+                              const int* nzc, int nnz, int* rows, int v) {
+  const int l = Warp::lane(), nw = 4 * nnz;
+  const uint32_t lt = (l == 31) ? 0x7fffffffu : ((1u << l) - 1u);
+  int n = 0;
+  for (int d0 = 0; d0 < P; d0 += Warp::NL) {
+    const int d = d0 + l;
+    const int has = d < P && test_bit(anc + (uint32_t)d * (uint32_t)Ws, c);
+    const uint32_t mask = Warp::ballot(has);
+    if (has) rows[n + popc32(mask & lt)] = d;
+    n += popc32(mask);
+  }
+  Warp::sync();
+  for (int i = l; i < n * nw; i += Warp::NL) {
+    const int r = i / nw, k = i - r * nw, d = rows[r];
+    const int wd = 4 * nzc[1 + (k >> 2)] + (k & 3);  // word of the row
+    uint32_t b = Lw[wd] & ~anc[(uint32_t)d * (uint32_t)Ws + wd];
+    int* out = anc_freq + (int64_t)d * P + 32 * wd;
+    while (b) {
+      int idx[8], x[8];
+#pragma unroll
+      for (int t = 0; t < 8; t++) { idx[t] = b ? ffs32(b) - 1 : -1; b &= b - 1u; }
+#pragma unroll
+      for (int t = 0; t < 8; t++) if (idx[t] >= 0) x[t] = out[idx[t]];
+#pragma unroll
+      for (int t = 0; t < 8; t++) if (idx[t] >= 0) out[idx[t]] = x[t] + v;
+    }
+  }
+  Warp::sync();
+}
+BN_HD void anc_tab_rows(const ChainParams& p, const ChainMem& m, int c, const DelLayout& lay, int nnz, int v) {
+  anc_tab_flip(m.anc, p.Ws, p.P, m.anc_freq, c, (const uint32_t*)lay.L, lay.nzc, nnz, lay.lists, v);
+}
+
+// accepted addition j -> c, BEFORE anc_after_add: the bits N = anc(j) & ~anc(c) that rows of {c} u desc(c)
+// gain turn on at iteration first_counted (v = -max(t, drop)).  N = 0: a redundant edge, nothing changes.
+BN_HD void anc_tab_add(const ChainParams& p, const ChainMem& m, int j, int c, int v) {
+  const RowGeom g = row_geom(p);
+  const int l = Warp::lane();
+  const DelLayout lay = anc_tab_layout(p, m);
+  const U4* aj = (const U4*)(m.anc + (uint32_t)j * (uint32_t)p.Ws);
+  const U4* ac = (const U4*)(m.anc + (uint32_t)c * (uint32_t)p.Ws);
+  const uint32_t lt = (l == 31) ? 0x7fffffffu : ((1u << l) - 1u);
+  int nnz = 0;
+  for (int ch0 = 0; ch0 < g.chunks; ch0 += Warp::NL) {
+    const int ch = ch0 + l;
+    U4 n = {0u, 0u, 0u, 0u};
+    if (ch < g.chunks) n = andn4(aj[ch], ac[ch]);
+    const int nz = nz4(n);
+    const uint32_t mask = Warp::ballot(nz);
+    if (nz) { lay.L[ch] = n; lay.nzc[1 + nnz + popc32(mask & lt)] = ch; }
+    nnz += popc32(mask);
+  }
+  Warp::sync();
+  if (nnz) anc_tab_rows(p, m, c, lay, nnz, v);
+}
+
+// accepted deletion at c, AFTER anc_after_delete changed rows (s.anc_changed): the bits of L that rows of
+// {c} u desc(c) no longer hold turn off (v = +max(t, drop)).  anc_del_team reads L and nzc but never
+// writes them, so they are still those of this deletion.
+BN_HD void anc_tab_del(const ChainParams& p, const ChainMem& m, int c, int v) {
+  const DelLayout lay = anc_tab_layout(p, m);
+  anc_tab_rows(p, m, c, lay, lay.nzc[0], v);
+}
+
 // empty graph: every row holds its own node only
 BN_HD void anc_reset(const ChainParams& p, ChainMem& m) {
   const int l = Warp::lane();
@@ -930,6 +1035,7 @@ BN_HD void chain_init(const ChainParams& p, ChainMem& m, ChainScalars& s, RngStr
   if (random) { /* ancestor rows were kept while the graph was drawn */ }
   else if (s.te_true > 0) anc_build_all(p, m);
   else anc_reset(p, m);
+  if (m.anc_freq) anc_tab_all(p, m, -counted_from);  // the start graph's paths are counted from max(drop, iter)
   // base scores (and the per-node factors of the MaxPar > 8 kernels), or those of the stopped run:
   // after a Givens downdate (MaxPar > 8) they differ from a fresh factorisation in the last bits
   s.n_nonpd = 0;
@@ -1829,6 +1935,7 @@ BN_HD void apply_move_vals(const ChainParams& p, ChainMem& m, ChainScalars& s, i
     s.te_true++; s.agree_true += ag;
     Warp::sync();
     const long long tq1 = cycle_now();
+    if (m.anc_freq) anc_tab_add(p, m, j, c, -(int)first_counted);  // (reads the rows before the update)
     anc_after_add(p, m, j, c, s.anc_changed);
     (void)tq1;
   } else {
@@ -1865,6 +1972,7 @@ BN_HD void apply_move_vals(const ChainParams& p, ChainMem& m, ChainScalars& s, i
 #else
     anc_after_delete(p, m, c, s.anc_changed);
 #endif
+    if (m.anc_freq && s.anc_changed) anc_tab_del(p, m, c, (int)first_counted);
     s.cyc[9] += tq1 - tq0; s.cyc[10] += cycle_now() - tq1;
   }
   if (KMAX > 8 && type == 1 && newrow) {
@@ -2434,6 +2542,10 @@ BN_HD void run_chain(const ChainParams& p, ChainMem& m, ChainScalars& s, RngStre
         if (cnt > 0) m.edge_freq[(int64_t)m.par[(int64_t)c * p.max_par + e] + (int64_t)c * p.P] += (int)cnt;
       }
     }
+  }
+  if (m.anc_freq) {
+    Warp::sync();
+    anc_tab_all(p, m, p.n_iter > p.drop ? p.n_iter : p.drop);  // the paths of the final graph, up to the end
   }
   Warp::sync();
 }

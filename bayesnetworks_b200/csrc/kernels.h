@@ -7,7 +7,9 @@
 
 namespace bn {
 
-struct ChainWorkspace {  // arrays over all chains of a run (device memory)
+// (a kernel parameter: 16-byte aligned, so that a new field shifts the parameters behind it by whole 16-byte
+// steps and the default kernels keep their code)
+struct alignas(16) ChainWorkspace {  // arrays over all chains of a run (device memory)
   int* par; int* npar; int* born; double* base;
   int* hp_list;
   uint32_t* anc; uint32_t* haspar;   // anc rows are anc_stride(W) words apart in global memory
@@ -25,7 +27,10 @@ struct ChainWorkspace {  // arrays over all chains of a run (device memory)
   const ChainStart* start;             // [nc] resumed chains: each runs n_iter iterations from its start->iter
   int scores_in;                       // base (and fac) already hold the chains' scores and factors
   int scores_out;                      // write the final scores back to base when they lived in shared memory
-  int with_state;                      // any of the above, or the chains' end state wanted: the WITH_STATE kernels
+  int with_state;                      // any of the above, the chains' end state wanted, or anc_freq: the
+                                       // WITH_STATE kernels
+  int* anc_freq;                       // [nc][P][P] posterior ancestor tabulation, or null (last: the fields the
+                                       // default kernels read keep their offsets)
 };
 
 // Which per-chain arrays live in dynamic shared memory (byte offset, -1 = global memory).

@@ -70,3 +70,22 @@ def summarize_result(result, graph, max_par: int, n_iter: int, drop: int = 0) ->
     """``summarize`` for a :class:`~bayesnetworks_b200.api.ChainResult` run with ``tabulate=True``."""
     return summarize(result.proposed, result.reject, result.npar_freq, result.edge_freq, graph.source, graph.target,
                      result.final_parents, result.final_npar, max_par, n_counted=max(n_iter - drop, 0))
+
+
+def ancestor_posterior(results) -> np.ndarray:
+    """Posterior probability of a directed path, [descendant, ancestor], pooled over chains.
+
+    ``results``: :class:`~bayesnetworks_b200.api.ChainResult` objects run with ``tabulate_ancestors=True``,
+    or their ``anc_freq`` arrays (segments of resumed runs may be listed alongside: counts add up).  The
+    counts are summed in int64 and each row is divided by the pooled diagonal, the number of tabulated
+    iterations; entry [d, a] is the share of them in which a is an ancestor of d (the diagonal is 1).
+    Rows without tabulated iterations are NaN."""
+    arrs = [np.asarray(getattr(r, "anc_freq", r)) for r in results]
+    if not arrs or any(a is None or a.ndim != 2 or a.shape[0] != a.shape[1] for a in arrs):
+        raise ValueError("ancestor_posterior needs [P, P] anc_freq arrays (run with tabulate_ancestors=True)")
+    total = np.zeros(arrs[0].shape, dtype=np.int64)
+    for a in arrs:
+        total += a
+    n = np.diagonal(total).astype(np.float64)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        return total / n[:, None]

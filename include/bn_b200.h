@@ -233,7 +233,7 @@ typedef struct bn_run_args {
   int* moves;              /* [n_chains*moves_capacity*4] */
   /* posterior tabulation (optional, may be NULL), Bayes-networks/main.cpp:289-297:
      edge_freq[chain][parent + child*P] += 1 for every edge of the kept graph after each
-     iteration i with i+1 > drop */
+     iteration i with i+1 > drop (anc_freq, at the end of this struct, tabulates directed paths the same way) */
   int* edge_freq;
   /* freqNpar of the same Tabulate(), main.cpp:291 (optional, may be NULL; ABI version >= 2):
      npar_freq[chain][node*(max_par+1) + k] = counted iterations the node spent with k parents */
@@ -277,6 +277,18 @@ typedef struct bn_run_args {
   bn_chain_state* state_out;
   const double* score_state_in;
   double* score_state_out;
+  /* ---- posterior ancestor tabulation (optional, may be NULL; host or device memory as device_outputs says) ----
+     anc_freq[chain][a + d*P] counts the iterations i with i+1 > drop after which the kept graph has a
+     directed path a -> ... -> d (a is an ancestor of d): the iterations and graphs edge_freq counts, from
+     max(drop, iter) on, with the same index orientation, edge_freq[parent + child*P].  So
+       - the diagonal holds the number of tabulated iterations (a node is its own ancestor): the
+         denominator of the posterior probability of a path;
+       - anc_freq >= edge_freq elementwise.
+     Like edge_freq it covers the iterations of this call only; the segments of a resumed run add up to
+     the uninterrupted run's counts, and bn_chain_state carries nothing for it.  The chains run the
+     kernels of the resumable-chain fields (the two-CTA form is not used); every other output is the
+     same as without it.  P*P ints per chain, as edge_freq. */
+  int* anc_freq;
 } bn_run_args;
 
 /* Per-chain length (doubles) of score_state_in / score_state_out. */
