@@ -66,7 +66,14 @@ class RunArgs(C.Structure):
                 ("moves_capacity", C.c_int), ("n_moves", _ip), ("moves", _ip), ("edge_freq", _ip),
                 ("npar_freq", _ip), ("mt_state_in", _ip), ("mt_state_out", _ip),
                 ("start_parents", _ip), ("start_n_par", _ip), ("state_in", C.c_void_p), ("state_out", C.c_void_p),
-                ("score_state_in", _dp), ("score_state_out", _dp), ("anc_freq", _ip)]
+                ("score_state_in", _dp), ("score_state_out", _dp), ("anc_freq", _ip),
+                ("best_parents", _ip), ("best_n_par", _ip), ("best", C.c_void_p)]
+
+
+class BestGraphC(C.Structure):
+    """bn_best_graph"""
+    _fields_ = [("log_post", C.c_double), ("log_lik", C.c_double), ("log_prior", C.c_double),
+                ("iter", C.c_int64), ("total_edges", C.c_int), ("found", C.c_int)]
 
 
 class ChainStateC(C.Structure):

@@ -49,11 +49,36 @@ class ChainResult:
     mt_state: Optional[np.ndarray] = None        # R-MT stream state after the run (.Random.seed[2:626])
     state: Optional["ChainState"] = None         # run(want_state=True): where the chain continues from
     anc_freq: Optional[np.ndarray] = None        # [descendant, ancestor] counts of directed paths (tabulate_ancestors)
+    best: Optional["BestGraph"] = None           # run(track_best=True): the best graph the chain visited
 
     def edges(self):
         """(parent, child) pairs, 0-based, per-child list order."""
         return [(int(self.final_parents[c, e]), c)
                 for c in range(len(self.final_npar)) for e in range(int(self.final_npar[c]))]
+
+
+@dataclass
+class BestGraph:
+    """The graph with the highest log posterior ``log_lik + log_prior`` among the graphs a chain held in
+    the iterations ``edge_freq`` counts (``Context.run(track_best=True)``; bn_best_graph of the C ABI).
+    ``log_lik`` is its globalLL, ``log_prior`` the chain's LogPrior of it; ``iter`` the first tabulated
+    iteration after which the chain held it.  ``found`` is False when the call tabulated no iteration:
+    the lists are then -1 / 0, the scores -inf and ``iter`` -1."""
+    parents: np.ndarray   # [P, max_par] int32, -1 padded, list order
+    npar: np.ndarray      # [P] int32
+    log_post: float
+    log_lik: float
+    log_prior: float
+    iter: int
+    found: bool
+
+    def edges(self):
+        """(parent, child) pairs, 0-based, per-child list order."""
+        return [(int(self.parents[c, e]), c) for c in range(len(self.npar)) for e in range(int(self.npar[c]))]
+
+    def as_start(self) -> "ChainState":
+        """A fresh chain from this graph (``Context.run(start=[...])``)."""
+        return ChainState.from_graph(self.parents, self.npar)
 
 
 _STATE_SCALARS = ("iter", "valid", "total_edges_member", "additions", "deletions", "uniforms")
@@ -352,7 +377,8 @@ class Context:
 
     def run(self, n_chains=1, n_iter=1000, output=100, initial_network=2, drop=0, rng="wh",
             seeds=None, replay=None, log_moves=False, moves_capacity=None, tabulate=False,
-            mt_state=None, want_mt_state=False, start=None, want_state=False, tabulate_ancestors=False):
+            mt_state=None, want_mt_state=False, start=None, want_state=False, tabulate_ancestors=False,
+            track_best=False):
         """Run ``n_chains`` independent chains; returns (list[ChainResult], kernel_ms).
 
         ``mt_state`` (rng="rmt"): R's stream state per chain, ``.Random.seed[2:626]`` (625 ints:
@@ -369,7 +395,12 @@ class Context:
         ``tabulate_ancestors``: ``ChainResult.anc_freq`` [descendant, ancestor] counts the tabulated
         iterations (those ``tabulate`` counts) after which the graph has a directed path ancestor -> ... ->
         descendant; its diagonal is the number of tabulated iterations.  Every other output is the same as
-        without it.  ``summary.ancestor_posterior`` pools chains into probabilities."""
+        without it.  ``summary.ancestor_posterior`` pools chains into probabilities.
+
+        ``track_best``: ``ChainResult.best`` is the :class:`BestGraph` of the chain, the highest log posterior
+        among the graphs held in the tabulated iterations of this call.  Every other output is the same as
+        without it.  ``summary.best_graph`` picks the best over chains, or over the segments of a resumed
+        run (the uninterrupted run's best)."""
         L = _lib.lib()
         kind = _RNG_KINDS[rng]
         p, mp = self.n_nodes, self.max_par
@@ -433,6 +464,13 @@ class Context:
         if tabulate_ancestors:
             afreq = np.zeros((n_chains, p, p), dtype=np.int32)
             args.anc_freq = afreq.ctypes.data_as(_lib._ip)
+        bpar = bnpar = bst = None
+        if track_best:
+            bpar = np.empty((n_chains, p, mp), dtype=np.int32)   # the library fills every entry
+            bnpar = np.empty((n_chains, p), dtype=np.int32)
+            bst = (_lib.BestGraphC * n_chains)()
+            args.best_parents, args.best_n_par = bpar.ctypes.data_as(_lib._ip), bnpar.ctypes.data_as(_lib._ip)
+            args.best = C.cast(bst, C.c_void_p)
         keep = []
         if start is not None:
             self._start_args(start, n_chains, kind, args, keep)
@@ -478,6 +516,11 @@ class Context:
                 edge_freq=None if freq is None else freq[ch],
                 npar_freq=None if nfreq is None else nfreq[ch],
                 anc_freq=None if afreq is None else afreq[ch]))
+            if bst is not None:
+                b = bst[ch]
+                out[-1].best = BestGraph(parents=bpar[ch], npar=bnpar[ch], log_post=float(b.log_post),
+                                         log_lik=float(b.log_lik), log_prior=float(b.log_prior), iter=int(b.iter),
+                                         found=bool(b.found))
             if st_out is not None:
                 o = st_out[ch]
                 out[-1].state = ChainState(

@@ -16,6 +16,15 @@
 
 using namespace bn;
 
+// bn_run copies the leading bn_best_graph out of each chain's BestTrack
+static_assert(offsetof(BestTrack, log_post) == offsetof(bn_best_graph, log_post) &&
+              offsetof(BestTrack, log_lik) == offsetof(bn_best_graph, log_lik) &&
+              offsetof(BestTrack, log_prior) == offsetof(bn_best_graph, log_prior) &&
+              offsetof(BestTrack, iter) == offsetof(bn_best_graph, iter) &&
+              offsetof(BestTrack, total_edges) == offsetof(bn_best_graph, total_edges) &&
+              offsetof(BestTrack, found) == offsetof(bn_best_graph, found) &&
+              sizeof(bn_best_graph) <= sizeof(BestTrack), "BestTrack must start with bn_best_graph");
+
 // ---------------------------------------------------------------------------
 // errors
 // ---------------------------------------------------------------------------
@@ -754,8 +763,13 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
     return fail(BN_ERR_BAD_ARG, "trace column pointer is NULL");
   // supplied start graphs and resumed chains
   const bool given = a->start_parents != nullptr, resume = a->state_in != nullptr;
-  // (the ancestor tabulation is compiled into the same kernels only: the default ones stay as they are)
-  const bool with_state = given || a->state_out || a->score_state_out || a->anc_freq;
+  // (the ancestor tabulation and the best-graph tracking are compiled into the same kernels only: the
+  // default ones stay as they are)
+  const bool with_state = given || a->state_out || a->score_state_out || a->anc_freq || a->best;
+  if (a->best_parents || a->best_n_par || a->best) {
+    const char* missing = !a->best_parents ? "best_parents" : !a->best_n_par ? "best_n_par" : !a->best ? "best" : nullptr;
+    if (missing) return fail(BN_ERR_BAD_ARG, "the best graph needs best_parents, best_n_par and best: %s is NULL", missing);
+  }
   if ((resume || a->score_state_in) && !given) return fail(BN_ERR_BAD_ARG, "state_in / score_state_in need start_parents");
   if (given && !a->start_n_par) return fail(BN_ERR_BAD_ARG, "start_parents needs start_n_par");
   if (resume && a->rng_kind == BN_RNG_RMT && !a->mt_state_in)
@@ -869,6 +883,25 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
     if (dev_out) w.anc_freq = a->anc_freq;
     else CU_TRY(buf.alloc(&w.anc_freq, (size_t)(nc * P * P)));
     CU_TRY(cudaMemsetAsync(w.anc_freq, 0, (size_t)(nc * P * P) * 4, c->stream));
+  }
+  int *best_par = nullptr, *best_npar = nullptr;
+  std::vector<BestTrack> best_setup;
+  if (a->best) {  // per chain: the lists (the output itself with device_outputs), the dirty set, the prior's constants
+    if (dev_out) { best_par = a->best_parents; best_npar = a->best_n_par; }
+    else { CU_TRY(buf.alloc(&best_par, (size_t)(nc * P * MP))); CU_TRY(buf.alloc(&best_npar, (size_t)(nc * P))); }
+    uint32_t* dirty = nullptr;
+    int* list = nullptr;
+    CU_TRY(buf.alloc(&dirty, (size_t)(nc * W)));
+    CU_TRY(buf.alloc(&list, (size_t)(nc * P)));
+    best_setup.resize(nc);
+    memset(best_setup.data(), 0, sizeof(BestTrack) * nc);
+    for (int ch = 0; ch < nc; ch++) {
+      BestTrack& b = best_setup[ch];
+      b.n_sim = c->n_sim_edges; b.phi = c->phi; b.omega = c->omega;
+      b.par = best_par + ch * P * MP; b.npar = best_npar + ch * P; b.dirty = dirty + ch * W; b.list = list + ch * P;
+    }
+    CU_TRY(buf.alloc(&w.best, (size_t)nc));  // (chain_init fills the rest)
+    CU_TRY(cudaMemcpyAsync(w.best, best_setup.data(), sizeof(BestTrack) * nc, cudaMemcpyHostToDevice, c->stream));
   }
   if (a->npar_freq) {
     if (dev_out) w.npar_freq = a->npar_freq;
@@ -1042,7 +1075,14 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
     if (a->edge_freq) CU_TRY(cudaMemcpy(a->edge_freq, w.edge_freq, (size_t)(nc * P * P) * 4, cudaMemcpyDeviceToHost));
     if (a->anc_freq) CU_TRY(cudaMemcpy(a->anc_freq, w.anc_freq, (size_t)(nc * P * P) * 4, cudaMemcpyDeviceToHost));
     if (a->npar_freq) CU_TRY(cudaMemcpy(a->npar_freq, w.npar_freq, (size_t)(nc * P * (MP + 1)) * 4, cudaMemcpyDeviceToHost));
+    if (a->best) {
+      CU_TRY(cudaMemcpy(a->best_parents, best_par, (size_t)(nc * P * MP) * 4, cudaMemcpyDeviceToHost));
+      CU_TRY(cudaMemcpy(a->best_n_par, best_npar, (size_t)(nc * P) * 4, cudaMemcpyDeviceToHost));
+    }
   }
+  if (a->best)  // the leading bn_best_graph of each chain's BestTrack
+    CU_TRY(cudaMemcpy2D(a->best, sizeof(bn_best_graph), w.best, sizeof(BestTrack), sizeof(bn_best_graph), nc,
+                        dev_out ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost));
   const cudaMemcpyKind fin_kind = dev_out ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
   if (final_parents) CU_TRY(cudaMemcpy(final_parents, w.par, (size_t)(nc * P * MP) * 4, fin_kind));
   if (final_n_par) CU_TRY(cudaMemcpy(final_n_par, w.npar, (size_t)(nc * P) * 4, fin_kind));

@@ -95,6 +95,26 @@ struct ChainStart {
   int acc_add, acc_del;  // accepted moves since `drop`
 };
 
+// Best graph visited (ChainMem.best; see best_visit), one per chain in global memory.  The first six fields
+// are bn_best_graph of include/bn_b200.h, which bn_run copies out; then the tracking state; then what the
+// caller sets up (so that the chain itself carries one pointer for it).
+struct BestTrack {
+  double log_post, log_lik, log_prior;
+  int64_t iter;          // first tabulated iteration after which the chain held the best graph (-1: none)
+  int total_edges;
+  int found;             // 0: no graph was a candidate yet
+  int64_t from;          // D = max(drop, start iteration): a graph left at an iteration > D is a candidate
+  int64_t born;          // iteration of the move that created the current graph (the start iteration at first)
+  int n_dirty;           // length of list
+  // set by the caller
+  int n_sim;             // NsimEdges
+  double phi, omega;
+  int* par;              // [P][max_par] the best graph's lists: valid for every node outside the dirty set
+  int* npar;             // [P]
+  uint32_t* dirty;       // [W] nodes whose list changed since par / npar were last synchronised
+  int* list;             // [P] the same set as a list, in marking order
+};
+
 struct ChainMem {  // per-chain global memory
   int* par;            // [P][max_par] ordered parent lists (edges[child])
   int* npar;           // [P]
@@ -128,6 +148,8 @@ struct ChainMem {  // per-chain global memory
   const double* base_in = nullptr;    // [P] scores to start from; with it fac already holds the factors (MaxPar > 8)
   // posterior ancestor tabulation (anc_tab_*; null: off)
   int* anc_freq = nullptr;            // [ancestor + descendant*P] iterations with a directed path ancestor -> descendant
+  // best graph visited (best_*; null: off)
+  BestTrack* best = nullptr;
 };
 
 struct ChainScalars {  // lives in registers (warp-uniform)
@@ -891,6 +913,97 @@ BN_HD void anc_tab_del(const ChainParams& p, const ChainMem& m, int c, int v) {
   anc_tab_rows(p, m, c, lay, lay.nzc[0], v);
 }
 
+// Lane l sums p = l, l+32, ... ascending, then a fixed-order tree: deterministic (sum_base: globalLL).
+BN_HD double sum_scores(const double* base, int P) {
+  double acc = 0.0;
+  for (int c = Warp::lane(); c < P; c += Warp::NL) acc += base[c];
+  return Warp::sum(acc);
+}
+
+// ---------------------------------------------------------------------------
+// Best graph visited (ChainMem.best): the graph with the highest log_lik + log_prior among the graphs
+// edge_freq counts.  With D = max(drop, iter0), a graph created at iteration t and replaced at t' (or held
+// to the end of the call) is counted iff t' > D (end > D).  log_lik is the graph's globalLL (sum_scores of
+// the score cache); log_prior is prior_value of its FP + FN and TotalEdges.  A later graph replaces the best
+// only when strictly greater: the first to reach the maximum wins.  Its `iter` is max(t, D).
+// No copy of the graph per new best: BestTrack.par / npar equal the current lists of every node outside
+// the dirty set, whose members are the nodes accepted moves changed since the last new best.  A new best
+// copies the dirty nodes' lists and empties the set; so par / npar always hold the best graph.
+// ---------------------------------------------------------------------------
+BN_HD void best_init(const ChainParams& p, const ChainMem& m, int64_t it0, int64_t from) {
+  const int l = Warp::lane(), MP = p.max_par;
+  BestTrack& b = *m.best;
+  for (int64_t i = l; i < (int64_t)p.P * MP; i += Warp::NL) b.par[i] = m.par[i];
+  for (int i = l; i < p.P; i += Warp::NL) b.npar[i] = m.npar[i];
+  for (int w = l; w < p.W; w += Warp::NL) b.dirty[w] = 0u;
+  Warp::sync();
+  if (l == 0) {
+    b.log_post = b.log_lik = b.log_prior = -INFINITY;
+    b.iter = -1; b.total_edges = 0; b.found = 0;
+    b.from = from; b.born = it0; b.n_dirty = 0;
+  }
+  Warp::sync();
+}
+
+// The current graph is about to be left after iteration `it` (c >= 0: an accepted move at node c, called
+// before it changes anything) or held at the end of the call (c = -1, it = end).  With it > D the graph is a
+// candidate: its log_lik is *gll when gll_ok, else sum_scores, left in *gll (returns 1 then: the caller keeps
+// it as its globalLL, the graph has not changed).  Not inlined: resumable runs without the tracking keep
+// the instruction-cache footprint of their chain loop.
+BN_NOINLINE int best_visit(BestTrack* bt, const double* base, const int* par, const int* npar, int P, int MP,
+                           int te, int ag, int64_t it, int c, int gll_ok, double* gll) {
+  const int l = Warp::lane();
+  int computed = 0;
+  const int64_t D = bt->from;
+  int* bpar = bt->par; int* bnpar = bt->npar; uint32_t* dirty = bt->dirty; int* list = bt->list;
+  if (it > D) {
+    double ll = *gll;
+    if (!gll_ok) { ll = sum_scores(base, P); *gll = ll; computed = 1; }
+    const double lpr = prior_value(bt->phi, bt->omega, (te - ag) + (bt->n_sim - ag), te);
+    const double lp = add_rn(ll, lpr);
+    if (!bt->found || lp > bt->log_post) {
+      const int nd = bt->n_dirty;
+      for (int i = l; i < nd; i += Warp::NL) {
+        const int d = list[i];
+        bnpar[d] = npar[d];
+        for (int e = 0; e < MP; e++) bpar[(int64_t)d * MP + e] = par[(int64_t)d * MP + e];
+        dirty[d >> 5] = 0u;  // (every set bit of the word is a listed node)
+      }
+      Warp::sync();
+      if (l == 0) {
+        const int64_t born = bt->born;
+        bt->log_post = lp; bt->log_lik = ll; bt->log_prior = lpr;
+        bt->iter = born > D ? born : D; bt->total_edges = te; bt->found = 1;
+        bt->n_dirty = 0;
+      }
+      Warp::sync();
+    }
+  }
+  if (c >= 0 && l == 0) {  // c's list is about to change: the current graph is born at `it`
+    if (!test_bit(dirty, c)) { dirty[c >> 5] |= 1u << (c & 31); list[bt->n_dirty] = c; bt->n_dirty++; }
+    bt->born = it;
+  }
+  Warp::sync();
+  return computed;
+}
+
+BN_HD void best_check(const ChainParams& p, const ChainMem& m, ChainScalars& s, int64_t it, int c) {
+  double g = s.gll;
+  if (best_visit(m.best, m.base, m.par, m.npar, p.P, p.max_par, s.te_true, s.agree_true, it, c, s.gll_ok, &g)) {
+    s.gll = g; s.gll_ok = 1;
+  }
+}
+
+// end of the call: the final graph's turn, then -1 / 0 lists when no graph was a candidate (end <= D)
+BN_HD void best_finish(const ChainParams& p, const ChainMem& m, ChainScalars& s) {
+  best_check(p, m, s, p.n_iter, -1);
+  if (!m.best->found) {
+    for (int64_t i = Warp::lane(); i < (int64_t)p.P * p.max_par; i += Warp::NL) m.best->par[i] = -1;
+    for (int i = Warp::lane(); i < p.P; i += Warp::NL) m.best->npar[i] = 0;
+  }
+  Warp::sync();
+}
+
 // empty graph: every row holds its own node only
 BN_HD void anc_reset(const ChainParams& p, ChainMem& m) {
   const int l = Warp::lane();
@@ -1071,15 +1184,11 @@ BN_HD void chain_init(const ChainParams& p, ChainMem& m, ChainScalars& s, RngStr
   for (int t = 0; t < 6; t++) s.pw_cyc[t] = 0;
   for (int t = 0; t < 12; t++) s.cyc[t] = 0;
   s.slots_sim = 0;
+  if (m.best) best_init(p, m, it0, counted_from);  // the start graph is the current one, born at it0
 }
 
 // globalLL = sum_p score(p) of the kept graph (LogLikelihood(1), src/network.h:239-247).
-// Lane l sums p = l, l+32, ... ascending, then a fixed-order tree: deterministic.
-BN_HD double sum_base(const ChainParams& p, const ChainMem& m) {
-  double acc = 0.0;
-  for (int c = Warp::lane(); c < p.P; c += Warp::NL) acc += m.base[c];
-  return Warp::sum(acc);
-}
+BN_HD double sum_base(const ChainParams& p, const ChainMem& m) { return sum_scores(m.base, p.P); }
 
 // ---------------------------------------------------------------------------
 // Phase A: replay the draw order of `nslots` iterations (warp-uniform).
@@ -1884,6 +1993,7 @@ BN_HD void apply_move_vals(const ChainParams& p, ChainMem& m, ChainScalars& s, i
     if (bad) { s.status = 95; return; }
   }
 #endif
+  if (m.best) best_check(p, m, s, it, c);  // the graph left here, before anything changes
   int* pc = m.par + (int64_t)c * MP;
   int* bc = m.born ? m.born + (int64_t)c * MP : nullptr;  // (only read with edge_freq)
   const int k = m.npar[c];
@@ -2546,6 +2656,10 @@ BN_HD void run_chain(const ChainParams& p, ChainMem& m, ChainScalars& s, RngStre
   if (m.anc_freq) {
     Warp::sync();
     anc_tab_all(p, m, p.n_iter > p.drop ? p.n_iter : p.drop);  // the paths of the final graph, up to the end
+  }
+  if (m.best) {
+    Warp::sync();
+    best_finish(p, m, s);
   }
   Warp::sync();
 }

@@ -21,11 +21,11 @@ namespace bn {
 // ALL_SMEM: every per-chain array of the plan sits in dynamic shared memory, so the pointers
 // have a provable shared-memory provenance and the state accesses compile to LDS/STS
 // instead of generic loads.
-// WITH_STATE: the chains start from supplied graphs / resume states or export their state, or tabulate
-// ancestor relations (ChainWorkspace.with_state).  Without it the start pointers and anc_freq stay null
-// at compile time, so chain_init folds to the start of initial_network and the steady-state loop
-// compiles as it did before resumable chains existed (a per-chain end iteration would hold a register
-// for the whole loop).
+// WITH_STATE: the chains start from supplied graphs / resume states or export their state, tabulate
+// ancestor relations or track the best graph (ChainWorkspace.with_state).  Without it the start pointers,
+// anc_freq and best stay null at compile time, so chain_init folds to the start of initial_network and the
+// steady-state loop compiles as it did before resumable chains existed (a per-chain end iteration would
+// hold a register for the whole loop).
 template <int KMAX, bool ALL_SMEM, bool WITH_STATE>
 __global__ void __launch_bounds__((HELPER_WARPS + 1) * 32, 1) chain_kernel(ChainParams p, ChainWorkspace w, ChainRngArgs ra,
                                                    ChainSmemPlan sm, ChainResult* __restrict__ results) {
@@ -77,6 +77,7 @@ __global__ void __launch_bounds__((HELPER_WARPS + 1) * 32, 1) chain_kernel(Chain
     if (w.start) m.start = w.start + ch;
     if (w.scores_in) m.base_in = w.base + ch * P;
     if (w.anc_freq) m.anc_freq = w.anc_freq + ch * P * P;
+    if (w.best) m.best = w.best + ch;
   }
 
   RngStream rng;

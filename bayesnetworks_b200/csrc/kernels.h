@@ -27,10 +27,11 @@ struct alignas(16) ChainWorkspace {  // arrays over all chains of a run (device 
   const ChainStart* start;             // [nc] resumed chains: each runs n_iter iterations from its start->iter
   int scores_in;                       // base (and fac) already hold the chains' scores and factors
   int scores_out;                      // write the final scores back to base when they lived in shared memory
-  int with_state;                      // any of the above, the chains' end state wanted, or anc_freq: the
+  int with_state;                      // any of the above, the chains' end state wanted, anc_freq or best: the
                                        // WITH_STATE kernels
   int* anc_freq;                       // [nc][P][P] posterior ancestor tabulation, or null (last: the fields the
                                        // default kernels read keep their offsets)
+  BestTrack* best;                     // [nc] best graph visited (its arrays and constants set up by the caller), or null
 };
 
 // Which per-chain arrays live in dynamic shared memory (byte offset, -1 = global memory).

@@ -89,3 +89,21 @@ def ancestor_posterior(results) -> np.ndarray:
     n = np.diagonal(total).astype(np.float64)
     with np.errstate(invalid="ignore", divide="ignore"):
         return total / n[:, None]
+
+
+def best_graph(results):
+    """The best graph over chains of one run, or over the segments of a resumed chain listed in order.
+
+    ``results``: :class:`~bayesnetworks_b200.api.ChainResult` objects run with ``track_best=True``, or their
+    :class:`~bayesnetworks_b200.api.BestGraph`.  Returns the first of the highest ``log_post``, skipping those
+    with ``found`` False; None when none was found.  Over the segments of a resumed run this is the
+    uninterrupted run's best: a graph held across a boundary is a candidate in both segments, and the earlier
+    one wins the tie."""
+    best = None
+    for r in results:
+        b = getattr(r, "best", r)
+        if b is None or not hasattr(b, "log_post"):
+            raise ValueError("best_graph needs BestGraph objects (run with track_best=True)")
+        if b.found and (best is None or b.log_post > best.log_post):
+            best = b
+    return best

@@ -209,6 +209,14 @@ typedef struct bn_chain_state {
   int64_t uniforms;          /* uniforms consumed since iteration 0 (random start graph included) */
 } bn_chain_state;
 
+/* The best graph a chain visited in one call (bn_run_args.best). */
+typedef struct bn_best_graph {
+  double log_post, log_lik, log_prior;
+  int64_t iter;        /* first tabulated iteration after which the chain held it; -1 if none */
+  int total_edges;
+  int found;           /* 0: this call tabulated no iteration */
+} bn_best_graph;
+
 typedef struct bn_run_args {
   int n_chains;
   int rng_kind;            /* BN_RNG_* */
@@ -289,6 +297,30 @@ typedef struct bn_run_args {
      kernels of the resumable-chain fields (the two-CTA form is not used); every other output is the
      same as without it.  P*P ints per chain, as edge_freq. */
   int* anc_freq;
+  /* ---- best graph visited (optional: all three set, or none; host or device memory as device_outputs says) ----
+     For each chain, the graph with the highest log posterior log_lik + log_prior among the graphs edge_freq
+     counts: those kept after the iterations i with i+1 > drop, from max(drop, iter) up to the end of the
+     call.  With D = max(drop, iter), a graph created by the move at iteration t and replaced at iteration t'
+     (or held to the end) is a candidate iff t' > D (end > D); so the start graph is not one when the move at
+     iteration D is accepted, and it is the best when no move is accepted after D.
+       - log_lik is the chain's globalLL of that graph (the sum of its node scores in the chain's fixed order):
+         exactly the value a trace row logged while the graph was held shows.
+       - log_prior = -phi*(FP + FN) - omega*TotalEdges of that graph, FP = TotalEdges - Nagree and
+         FN = NsimEdges - Nagree (the chain's LogPrior, evaluated without contraction).
+       - Ties: a later graph replaces the best only if its log_post is strictly greater (the first graph to
+         reach the maximum wins).
+       - iter: the first tabulated iteration after which the chain held it, max(creation iteration, D).
+     When the call tabulates no iteration (end <= D): found = 0, the lists are -1 / 0, log_post, log_lik and
+     log_prior are -inf, iter = -1 and total_edges = 0.
+     Like edge_freq it covers the iterations of this call only and bn_chain_state carries nothing for it.
+     Segments of a resumed run combine on the host: the first of the highest log_post over the segments in
+     order, skipping found = 0, is the uninterrupted run's best (a graph held across a boundary is a candidate
+     in both segments and the earlier wins the tie); bit for bit when resumed with score_state_in.  The chains
+     run the kernels of the resumable-chain fields (the two-CTA form is not used); every other output is the
+     same as without it. */
+  int* best_parents;         /* [n_chains][P][max_par], -1 padded, list order */
+  int* best_n_par;           /* [n_chains][P] */
+  bn_best_graph* best;       /* [n_chains] */
 } bn_run_args;
 
 /* Per-chain length (doubles) of score_state_in / score_state_out. */
