@@ -21,7 +21,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "_obj")
 LIB = os.path.join(HERE, "libbn_b200.so")
 SOURCES = ["bn_api.cu", "gram.cu", "kernels.cu"]
-HEADERS = ["bn_common.cuh", "chain_core.cuh", "rng_core.cuh", "score_core.cuh", "gram.h", "kernels.h",
+HEADERS = ["bn_common.cuh", "chain_core.cuh", "rng_core.cuh", "score_core.cuh", "sweep_log.cuh", "gram.h", "kernels.h",
            os.path.join("..", "..", "include", "bn_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v"]

@@ -7,6 +7,7 @@
 
 #include "chain_core.cuh"
 #include "kernels.h"
+#include "sweep_log.cuh"
 
 namespace bn {
 
@@ -535,37 +536,6 @@ __device__ __forceinline__ void border_row(const double* __restrict__ C, int64_t
   }
 }
 
-// Natural logarithm for the sweep's addition loop (one per proposal; the kernel is bound by instruction
-// issue and libdevice's log is ~100 instructions): x = 2^e m with m in [sqrt(1/2), sqrt(2)),
-// log m = 2 atanh(s), s = (m - 1) / (m + 1), |s| <= 0.172, odd series to s^19 (truncation 2.4e-17 relative),
-// the reciprocal by __drcp_rn.  ~40 instructions, error below 2 ulp; the sweep's parity bar against the
-// oracle is 1e-9 relative.  The argument is a positive normal number at the call site (RSS above its floor times a
-// finite scale); anything else gives NaN.
-__device__ __forceinline__ double sweep_log(double x) {
-  int hi = __double2hiint(x);
-  const int lo = __double2loint(x);
-  if ((unsigned)(hi - 0x00100000) >= 0x7fe00000u) return __longlong_as_double(0x7ff8000000000000ll);  // (not a positive normal number)
-  int e = (hi >> 20) - 1023;
-  hi = (hi & 0x000fffff) | 0x3ff00000;
-  if (hi >= 0x3ff6a09e) { hi -= 0x00100000; e++; }  // m >= ~sqrt(2): halve
-  const double m = __hiloint2double(hi, lo);
-  const double f = m - 1.0;
-  const double s = f * __drcp_rn(2.0 + f);
-  const double s2 = s * s;
-  double p = 2.0 / 19.0;
-  p = fma(p, s2, 2.0 / 17.0);
-  p = fma(p, s2, 2.0 / 15.0);
-  p = fma(p, s2, 2.0 / 13.0);
-  p = fma(p, s2, 2.0 / 11.0);
-  p = fma(p, s2, 2.0 / 9.0);
-  p = fma(p, s2, 2.0 / 7.0);
-  p = fma(p, s2, 2.0 / 5.0);
-  p = fma(p, s2, 2.0 / 3.0);
-  const double de = (double)e;
-  // e ln2 + 2s + s^3 p, ln2 split so that e * ln2_hi is exact
-  return fma(de, 6.93147180369123816490e-01, fma(s * s2, p, fma(de, 1.90821492927058770002e-10, 2.0 * s)));
-}
-
 template <int KMAX, int SWEEP_WARPS>
 __global__ void __launch_bounds__(SWEEP_WARPS * 32, KMAX <= 8 ? 8 : 2) sweep_kernel(SweepParams sp) {
   constexpr int TRI = (KMAX + 1) * (KMAX + 2) / 2;  // augmented (k+1) lower triangle
@@ -630,6 +600,10 @@ __global__ void __launch_bounds__(SWEEP_WARPS * 32, KMAX <= 8 ? 8 : 2) sweep_ker
   if (!(rss > Ccc * RSS_FLOOR)) pd = false;
   const double base = pd ? -(n / 2.0) * log((rss / (n - (double)k - 1.0)) / syy) : -INFINITY;
   if (lane == 0 && sp.out_base) sp.out_base[wg] = base;
+  // an addition that leaves no residual degrees of freedom (k + 1 parents, N - k - 2 <= 0) scores -inf, as
+  // the chain's (N - 1) / (N - k - 2) = inf does (add_scale would be inf or negative and its log NaN): no RSS
+  // passes an infinite floor
+  const double add_floor = (k + 2 < sp.n_samples) ? Ccc * RSS_FLOOR : INFINITY;
 
   // prior bookkeeping of this graph
   const int te = sp.te[g], ag = sp.agree[g];
@@ -692,7 +666,7 @@ __global__ void __launch_bounds__(SWEEP_WARPS * 32, KMAX <= 8 ? 8 : 2) sweep_ker
             border_row<KMAX>(C, ldc, S, k, j, A, zrow, dj, ej);
           }
           const double rss_new = rss - ej * ej * __drcp_rn(dj);
-          if (dj > 0.0 && rss_new > Ccc * RSS_FLOOR) sc = neg_half_n * sweep_log(rss_new * add_scale);
+          if (dj > 0.0 && rss_new > add_floor) sc = neg_half_n * sweep_log(rss_new * add_scale);
           else sc = -INFINITY;   // not positive definite / an exact fit the Gram route cannot resolve
         }
         hr = sub_rn(add_rn(sub_rn(sc, base), a1 ? add_prior1 : add_prior0), old_prior);
