@@ -10,8 +10,9 @@ from .network import Network, create_network, read_dag, read_data  # noqa: F401
 from .api import (BestGraph, ChainResult, ChainState, Context, TRACE_COLUMNS, bn_mcmc, main_fun,  # noqa: F401
                   set_default_stream)
 from ._lib import BnError  # noqa: F401
-from .summary import ancestor_posterior, best_graph, summarize, summarize_result  # noqa: F401
+from .summary import (ancestor_posterior, best_graph, markov_blanket_posterior, summarize,  # noqa: F401
+                      summarize_result)
 
 __all__ = ["Network", "create_network", "read_dag", "read_data", "Context", "ChainResult", "ChainState",
            "TRACE_COLUMNS", "bn_mcmc", "main_fun", "BnError", "summarize", "summarize_result",
-           "ancestor_posterior", "BestGraph", "best_graph"]
+           "ancestor_posterior", "BestGraph", "best_graph", "markov_blanket_posterior"]

@@ -67,7 +67,7 @@ class RunArgs(C.Structure):
                 ("npar_freq", _ip), ("mt_state_in", _ip), ("mt_state_out", _ip),
                 ("start_parents", _ip), ("start_n_par", _ip), ("state_in", C.c_void_p), ("state_out", C.c_void_p),
                 ("score_state_in", _dp), ("score_state_out", _dp), ("anc_freq", _ip),
-                ("best_parents", _ip), ("best_n_par", _ip), ("best", C.c_void_p)]
+                ("best_parents", _ip), ("best_n_par", _ip), ("best", C.c_void_p), ("mb_freq", _ip)]
 
 
 class BestGraphC(C.Structure):

@@ -50,6 +50,7 @@ class ChainResult:
     state: Optional["ChainState"] = None         # run(want_state=True): where the chain continues from
     anc_freq: Optional[np.ndarray] = None        # [descendant, ancestor] counts of directed paths (tabulate_ancestors)
     best: Optional["BestGraph"] = None           # run(track_best=True): the best graph the chain visited
+    mb_freq: Optional[np.ndarray] = None         # [P, P] symmetric counts of Markov blanket pairs (tabulate_markov_blankets)
 
     def edges(self):
         """(parent, child) pairs, 0-based, per-child list order."""
@@ -378,7 +379,7 @@ class Context:
     def run(self, n_chains=1, n_iter=1000, output=100, initial_network=2, drop=0, rng="wh",
             seeds=None, replay=None, log_moves=False, moves_capacity=None, tabulate=False,
             mt_state=None, want_mt_state=False, start=None, want_state=False, tabulate_ancestors=False,
-            track_best=False):
+            track_best=False, tabulate_markov_blankets=False):
         """Run ``n_chains`` independent chains; returns (list[ChainResult], kernel_ms).
 
         ``mt_state`` (rng="rmt"): R's stream state per chain, ``.Random.seed[2:626]`` (625 ints:
@@ -400,7 +401,12 @@ class Context:
         ``track_best``: ``ChainResult.best`` is the :class:`BestGraph` of the chain, the highest log posterior
         among the graphs held in the tabulated iterations of this call.  Every other output is the same as
         without it.  ``summary.best_graph`` picks the best over chains, or over the segments of a resumed
-        run (the uninterrupted run's best)."""
+        run (the uninterrupted run's best).
+
+        ``tabulate_markov_blankets``: ``ChainResult.mb_freq`` [P, P] (symmetric) counts the tabulated iterations
+        after which j is in the Markov blanket of i: i -> j, j -> i, or a common child.  Its diagonal is the
+        number of tabulated iterations.  Every other output is the same as without it.
+        ``summary.markov_blanket_posterior`` pools chains into probabilities."""
         L = _lib.lib()
         kind = _RNG_KINDS[rng]
         p, mp = self.n_nodes, self.max_par
@@ -464,6 +470,10 @@ class Context:
         if tabulate_ancestors:
             afreq = np.zeros((n_chains, p, p), dtype=np.int32)
             args.anc_freq = afreq.ctypes.data_as(_lib._ip)
+        mbfreq = None
+        if tabulate_markov_blankets:
+            mbfreq = np.zeros((n_chains, p, p), dtype=np.int32)
+            args.mb_freq = mbfreq.ctypes.data_as(_lib._ip)
         bpar = bnpar = bst = None
         if track_best:
             bpar = np.empty((n_chains, p, mp), dtype=np.int32)   # the library fills every entry
@@ -515,7 +525,8 @@ class Context:
                 accepted_moves=None if moves is None else moves[ch, :int(n_moves[ch])],
                 edge_freq=None if freq is None else freq[ch],
                 npar_freq=None if nfreq is None else nfreq[ch],
-                anc_freq=None if afreq is None else afreq[ch]))
+                anc_freq=None if afreq is None else afreq[ch],
+                mb_freq=None if mbfreq is None else mbfreq[ch]))
             if bst is not None:
                 b = bst[ch]
                 out[-1].best = BestGraph(parents=bpar[ch], npar=bnpar[ch], log_post=float(b.log_post),

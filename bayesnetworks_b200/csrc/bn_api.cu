@@ -763,9 +763,9 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
     return fail(BN_ERR_BAD_ARG, "trace column pointer is NULL");
   // supplied start graphs and resumed chains
   const bool given = a->start_parents != nullptr, resume = a->state_in != nullptr;
-  // (the ancestor tabulation and the best-graph tracking are compiled into the same kernels only: the
-  // default ones stay as they are)
-  const bool with_state = given || a->state_out || a->score_state_out || a->anc_freq || a->best;
+  // (the ancestor and Markov blanket tabulations and the best-graph tracking are compiled into the same
+  // kernels only: the default ones stay as they are)
+  const bool with_state = given || a->state_out || a->score_state_out || a->anc_freq || a->best || a->mb_freq;
   if (a->best_parents || a->best_n_par || a->best) {
     const char* missing = !a->best_parents ? "best_parents" : !a->best_n_par ? "best_n_par" : !a->best ? "best" : nullptr;
     if (missing) return fail(BN_ERR_BAD_ARG, "the best graph needs best_parents, best_n_par and best: %s is NULL", missing);
@@ -902,6 +902,20 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
     }
     CU_TRY(buf.alloc(&w.best, (size_t)nc));  // (chain_init fills the rest)
     CU_TRY(cudaMemcpyAsync(w.best, best_setup.data(), sizeof(BestTrack) * nc, cudaMemcpyHostToDevice, c->stream));
+  }
+  int* mb_freq = nullptr;
+  std::vector<MbTrack> mb_setup;
+  if (a->mb_freq) {  // per chain: the counts (the output itself with device_outputs) and the witness matrix, both zeroed
+    uint16_t* wit = nullptr;
+    if (dev_out) mb_freq = a->mb_freq;
+    else CU_TRY(buf.alloc(&mb_freq, (size_t)(nc * P * P)));
+    CU_TRY(buf.alloc(&wit, (size_t)(nc * P * P)));
+    CU_TRY(cudaMemsetAsync(mb_freq, 0, (size_t)(nc * P * P) * 4, c->stream));
+    CU_TRY(cudaMemsetAsync(wit, 0, (size_t)(nc * P * P) * 2, c->stream));
+    mb_setup.resize(nc);
+    for (int ch = 0; ch < nc; ch++) { mb_setup[ch].freq = mb_freq + ch * P * P; mb_setup[ch].wit = wit + ch * P * P; }
+    CU_TRY(buf.alloc(&w.mb, (size_t)nc));
+    CU_TRY(cudaMemcpyAsync(w.mb, mb_setup.data(), sizeof(MbTrack) * nc, cudaMemcpyHostToDevice, c->stream));
   }
   if (a->npar_freq) {
     if (dev_out) w.npar_freq = a->npar_freq;
@@ -1074,6 +1088,7 @@ extern "C" int bn_run(bn_ctx* c, const bn_run_args* a, bn_trace* trace, int* fin
     if (mcap) CU_TRY(cudaMemcpy(a->moves, w.moves, (size_t)nc * mcap * 16, cudaMemcpyDeviceToHost));
     if (a->edge_freq) CU_TRY(cudaMemcpy(a->edge_freq, w.edge_freq, (size_t)(nc * P * P) * 4, cudaMemcpyDeviceToHost));
     if (a->anc_freq) CU_TRY(cudaMemcpy(a->anc_freq, w.anc_freq, (size_t)(nc * P * P) * 4, cudaMemcpyDeviceToHost));
+    if (a->mb_freq) CU_TRY(cudaMemcpy(a->mb_freq, mb_freq, (size_t)(nc * P * P) * 4, cudaMemcpyDeviceToHost));
     if (a->npar_freq) CU_TRY(cudaMemcpy(a->npar_freq, w.npar_freq, (size_t)(nc * P * (MP + 1)) * 4, cudaMemcpyDeviceToHost));
     if (a->best) {
       CU_TRY(cudaMemcpy(a->best_parents, best_par, (size_t)(nc * P * MP) * 4, cudaMemcpyDeviceToHost));

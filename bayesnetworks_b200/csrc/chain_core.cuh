@@ -115,6 +115,13 @@ struct BestTrack {
   int* list;             // [P] the same set as a list, in marking order
 };
 
+// Posterior Markov blanket tabulation (ChainMem.mb; see mb_pairs), one per chain in global memory, set up by
+// the caller (so that the chain itself carries one pointer for it).  Both matrices are symmetric.
+struct MbTrack {
+  int* freq;             // [i + j*P] iterations with (i, j) in the blanket (bn_run_args.mb_freq)
+  uint16_t* wit;         // [i + j*P] witnesses of the pair: the edge between i and j, and each common child
+};
+
 struct ChainMem {  // per-chain global memory
   int* par;            // [P][max_par] ordered parent lists (edges[child])
   int* npar;           // [P]
@@ -150,6 +157,8 @@ struct ChainMem {  // per-chain global memory
   int* anc_freq = nullptr;            // [ancestor + descendant*P] iterations with a directed path ancestor -> descendant
   // best graph visited (best_*; null: off)
   BestTrack* best = nullptr;
+  // posterior Markov blanket tabulation (mb_*; null: off)
+  MbTrack* mb = nullptr;
 };
 
 struct ChainScalars {  // lives in registers (warp-uniform)
@@ -1004,6 +1013,69 @@ BN_HD void best_finish(const ChainParams& p, const ChainMem& m, ChainScalars& s)
   Warp::sync();
 }
 
+// ---------------------------------------------------------------------------
+// Posterior Markov blanket tabulation (ChainMem.mb): freq[i + j*P] counts the iterations, from max(drop, iter)
+// on, after which i -> j, j -> i, or some node has both i and j as parents; the diagonal counts them all.
+// wit[i + j*P] holds the number of such reasons (the edge between i and j counts one, each common child one
+// more), so the pair is in the blanket iff wit > 0.  It is a function of the graph: an accepted move j -> c
+// changes the pairs (j, c) and (j, q), q a co-parent, by one witness each (mb_move).  The count accumulates
+// with signs, as anc_freq does: a pair that enters the blanket at iteration t subtracts max(t, drop), one that
+// leaves adds it.  The chain start adds the start graph's nodes one by one (mb_graph, -max(drop, iter)) and the
+// end removes them all again (+max(end, drop)), so no pass over all P * P pairs is needed.
+// ---------------------------------------------------------------------------
+BN_HD void mb_count(int* x, int v) {
+#if defined(__CUDA_ARCH__)
+  atomicAdd(x, v);  // (result unused: a reduction the lane does not wait for; the lanes' pairs are distinct)
+#else
+  *x += v;
+#endif
+}
+
+// One witness more (dw = +1) or less (dw = -1) for each pair listed; a count that leaves or reaches 0 adds
+// -dw * v to both halves of the pair.  j >= 0: the pairs (j, pc[0..k)) and (j, c) of a move j -> c.  j < 0: every
+// witness node c holds, the pairs (pc[e], pc[f]) for f < e < k and (pc[e], c).  The pairs of one call are
+// distinct, so lanes own distinct counters.  Not inlined: resumable runs without the tabulation keep the
+// registers and instruction-cache footprint of their chain loop.
+BN_NOINLINE void mb_pairs(MbTrack* mt, int P, int c, const int* pc, int k, int j, int dw, int v) {
+  int* freq = mt->freq;
+  uint16_t* wit = mt->wit;
+  const int n = j >= 0 ? k + 1 : k * (k + 1) / 2;
+  for (int t = Warp::lane(); t < n; t += Warp::NL) {
+    int a, b;
+    if (j >= 0) {
+      a = j; b = t < k ? pc[t] : c;
+    } else {  // row e of the triangle: (pc[e], pc[0..e)), then (pc[e], c)
+      int e = 0;
+      while ((e + 1) * (e + 2) / 2 <= t) e++;
+      const int f = t - e * (e + 1) / 2;
+      a = pc[e]; b = f < e ? pc[f] : c;
+    }
+    const int64_t ab = (int64_t)a + (int64_t)b * P, ba = (int64_t)b + (int64_t)a * P;
+    const int w0 = wit[ab], w1 = w0 + dw;
+    wit[ab] = (uint16_t)w1; wit[ba] = (uint16_t)w1;
+    if (w0 == 0 || w1 == 0) { mb_count(freq + ab, -dw * v); mb_count(freq + ba, -dw * v); }
+  }
+  Warp::sync();
+}
+
+// accepted move j -> c (v = first_counted): an addition with c's list before j is appended, a deletion with the
+// list after the shift (dw = +1 / -1)
+BN_HD void mb_move(const ChainParams& p, const ChainMem& m, int c, int k, int j, int dw, int v) {
+  mb_pairs(m.mb, p.P, c, m.par + (int64_t)c * p.max_par, k, j, dw, v);
+}
+
+// every node's witnesses added (chain start, dw = +1, v = max(drop, iter)) or removed (end, dw = -1,
+// v = max(end, drop)); the diagonal counts the same iterations (-dw * v).  The nodes go one at a time: two
+// nodes may share a pair.
+BN_HD void mb_graph(const ChainParams& p, const ChainMem& m, int dw, int v) {
+  for (int c = 0; c < p.P; c++) {
+    const int k = m.npar[c];
+    if (k) mb_pairs(m.mb, p.P, c, m.par + (int64_t)c * p.max_par, k, -1, dw, v);
+  }
+  for (int i = Warp::lane(); i < p.P; i += Warp::NL) m.mb->freq[(int64_t)i * (p.P + 1)] += -dw * v;
+  Warp::sync();
+}
+
 // empty graph: every row holds its own node only
 BN_HD void anc_reset(const ChainParams& p, ChainMem& m) {
   const int l = Warp::lane();
@@ -1149,6 +1221,7 @@ BN_HD void chain_init(const ChainParams& p, ChainMem& m, ChainScalars& s, RngStr
   else if (s.te_true > 0) anc_build_all(p, m);
   else anc_reset(p, m);
   if (m.anc_freq) anc_tab_all(p, m, -counted_from);  // the start graph's paths are counted from max(drop, iter)
+  if (m.mb) mb_graph(p, m, 1, counted_from);         // and its blanket pairs
   // base scores (and the per-node factors of the MaxPar > 8 kernels), or those of the stopped run:
   // after a Givens downdate (MaxPar > 8) they differ from a fresh factorisation in the last bits
   s.n_nonpd = 0;
@@ -2046,6 +2119,7 @@ BN_HD void apply_move_vals(const ChainParams& p, ChainMem& m, ChainScalars& s, i
     Warp::sync();
     const long long tq1 = cycle_now();
     if (m.anc_freq) anc_tab_add(p, m, j, c, -(int)first_counted);  // (reads the rows before the update)
+    if (m.mb) mb_move(p, m, c, k, j, 1, (int)first_counted);        // (c's list before j: pc[0..k))
     anc_after_add(p, m, j, c, s.anc_changed);
     (void)tq1;
   } else {
@@ -2076,6 +2150,7 @@ BN_HD void apply_move_vals(const ChainParams& p, ChainMem& m, ChainScalars& s, i
     }
     s.te_true--; s.agree_true -= ag;
     Warp::sync();
+    if (m.mb) mb_move(p, m, c, k - 1, j, -1, (int)first_counted);  // (c's list after the shift)
     const long long tq1 = cycle_now();
 #if defined(BN_PHASE_CYCLES)
     anc_after_delete(p, m, c, s.anc_changed, s.cyc);   // [6] collect+clear, [7] first barrier, [8] round work, [11] round barriers
@@ -2656,6 +2731,10 @@ BN_HD void run_chain(const ChainParams& p, ChainMem& m, ChainScalars& s, RngStre
   if (m.anc_freq) {
     Warp::sync();
     anc_tab_all(p, m, p.n_iter > p.drop ? p.n_iter : p.drop);  // the paths of the final graph, up to the end
+  }
+  if (m.mb) {
+    Warp::sync();
+    mb_graph(p, m, -1, p.n_iter > p.drop ? p.n_iter : p.drop);  // the blanket pairs of the final graph
   }
   if (m.best) {
     Warp::sync();

@@ -23,10 +23,10 @@ namespace bn {
 // have a provable shared-memory provenance and the state accesses compile to LDS/STS
 // instead of generic loads.
 // WITH_STATE: the chains start from supplied graphs / resume states or export their state, tabulate
-// ancestor relations or track the best graph (ChainWorkspace.with_state).  Without it the start pointers,
-// anc_freq and best stay null at compile time, so chain_init folds to the start of initial_network and the
-// steady-state loop compiles as it did before resumable chains existed (a per-chain end iteration would
-// hold a register for the whole loop).
+// ancestor relations or Markov blankets, or track the best graph (ChainWorkspace.with_state).  Without it the
+// start pointers, anc_freq, best and mb stay null at compile time, so chain_init folds to the start of
+// initial_network and the steady-state loop compiles as it did before resumable chains existed (a per-chain
+// end iteration would hold a register for the whole loop).
 template <int KMAX, bool ALL_SMEM, bool WITH_STATE>
 __global__ void __launch_bounds__((HELPER_WARPS + 1) * 32, 1) chain_kernel(ChainParams p, ChainWorkspace w, ChainRngArgs ra,
                                                    ChainSmemPlan sm, ChainResult* __restrict__ results) {
@@ -79,6 +79,7 @@ __global__ void __launch_bounds__((HELPER_WARPS + 1) * 32, 1) chain_kernel(Chain
     if (w.scores_in) m.base_in = w.base + ch * P;
     if (w.anc_freq) m.anc_freq = w.anc_freq + ch * P * P;
     if (w.best) m.best = w.best + ch;
+    if (w.mb) m.mb = w.mb + ch;
   }
 
   RngStream rng;

@@ -107,3 +107,23 @@ def best_graph(results):
         if b.found and (best is None or b.log_post > best.log_post):
             best = b
     return best
+
+
+def markov_blanket_posterior(results) -> np.ndarray:
+    """Posterior probability that j is in the Markov blanket of i (i -> j, j -> i, or a common child), [i, j],
+    pooled over chains.
+
+    ``results``: :class:`~bayesnetworks_b200.api.ChainResult` objects run with ``tabulate_markov_blankets=True``,
+    or their ``mb_freq`` arrays (segments of resumed runs may be listed alongside: counts add up).  The counts
+    are summed in int64 and each row is divided by the pooled diagonal, the number of tabulated iterations;
+    the result is symmetric and its diagonal is 1.  Rows without tabulated iterations are NaN."""
+    arrs = [np.asarray(getattr(r, "mb_freq", r)) for r in results]
+    if not arrs or any(a is None or a.ndim != 2 or a.shape[0] != a.shape[1] for a in arrs):
+        raise ValueError("markov_blanket_posterior needs [P, P] mb_freq arrays "
+                         "(run with tabulate_markov_blankets=True)")
+    total = np.zeros(arrs[0].shape, dtype=np.int64)
+    for a in arrs:
+        total += a
+    n = np.diagonal(total).astype(np.float64)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        return total / n[:, None]

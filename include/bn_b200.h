@@ -246,7 +246,8 @@ typedef struct bn_run_args {
   int* moves;              /* [n_chains*moves_capacity*4] */
   /* posterior tabulation (optional, may be NULL), Bayes-networks/main.cpp:289-297:
      edge_freq[chain][parent + child*P] += 1 for every edge of the kept graph after each
-     iteration i with i+1 > drop (anc_freq, at the end of this struct, tabulates directed paths the same way) */
+     iteration i with i+1 > drop (anc_freq and mb_freq, at the end of this struct, tabulate directed paths and
+     Markov blankets the same way) */
   int* edge_freq;
   /* freqNpar of the same Tabulate(), main.cpp:291 (optional, may be NULL; ABI version >= 2):
      npar_freq[chain][node*(max_par+1) + k] = counted iterations the node spent with k parents */
@@ -326,6 +327,19 @@ typedef struct bn_run_args {
   int* best_parents;         /* [n_chains][P][max_par], -1 padded, list order */
   int* best_n_par;           /* [n_chains][P] */
   bn_best_graph* best;       /* [n_chains] */
+  /* ---- posterior Markov blanket tabulation (optional, may be NULL; host or device memory as device_outputs says) ----
+     mb_freq[chain][i + j*P] counts the iterations i' with i'+1 > drop after which j is in the Markov blanket of i
+     in the kept graph: i -> j, j -> i, or some node has both i and j as parents.  These are the iterations and
+     graphs edge_freq counts, from max(drop, iter) on.  So
+       - the matrix is symmetric, and its diagonal holds the number of tabulated iterations: the denominator
+         of the posterior probability of blanket membership;
+       - off the diagonal, mb_freq >= edge_freq + its transpose, with equality at max_par = 1.
+     Like edge_freq it covers the iterations of this call only; the segments of a resumed run add up to
+     the uninterrupted run's counts, and bn_chain_state carries nothing for it.  The chains run the
+     kernels of the resumable-chain fields (the two-CTA form is not used); every other output is the
+     same as without it.  P*P ints per chain, as edge_freq, and a P*P matrix of 16-bit witness counts per
+     chain in scratch memory. */
+  int* mb_freq;
 } bn_run_args;
 
 /* Per-chain length (doubles) of score_state_in / score_state_out. */
